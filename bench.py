@@ -12,6 +12,11 @@ once, outside the timed region - the regime of the reference's own harness, demo
 edges/sec = (2 * E) / step time: every layer pass streams all E input edges (appended self loops are NOT counted).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config headline|cfg1..cfg5] [--scale S]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes the arrays the last timed step returned as DIR/<name>.npy (float32), so that two builds can be
+compared output for output on identical seeded inputs; an output above its share of 64 MB is stored as a fixed sample of
+its rows (see dump_outputs).  Single-GPU configs of --impl ours only.
 
 --config selects one of BASELINE.json's configs (default: headline = the configuration the metric is quoted on); every
 config prints the same JSON contract with its own roofline.  --gpus N > 1 (under torchrun) runs the headline step
@@ -73,6 +78,8 @@ def parse_args():
                     help="reference arm: graph scaled down by this factor (0 = auto: about two minutes of CPU work in total)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     return ap.parse_args()
 
 
@@ -413,7 +420,8 @@ NCU_TRAFFIC = {"gat": 128185916000, "spmm_d128": 63372534000}
 
 def build_workload(args, tfg, device):
     """Graph, features, layers and the step function of args.config on one GPU.  Returns a dict with: x_host, step,
-    E, passes, kernels = {family: (abi call, algorithmic bytes per step, description)}."""
+    outputs (a name for each array the step returns), E, passes, kernels = {family: (abi call, algorithmic bytes per
+    step, description)}."""
     cfg, n, pairs = config_sizes(args)
     F = cfg["features"]
     kind = cfg["kind"]
@@ -449,6 +457,7 @@ def build_workload(args, tfg, device):
             kernels["gat_projections"] = ("tfgk_gemm_proj_f32", proj_bytes(3 * UNITS),
                                           "gemm_proj_ts_kernel<STAGES>, Q|K|V in one launch (tfgk_gemm_proj_f32)", None)
         step = lambda xd: tuple(f(xd) for f in layers)     # noqa: E731
+        outputs = tuple(k for k in ("gcn", "gat") if k in kind)
         passes = len(layers)
     elif kind == "gcn2":
         # sparse bag-of-words features like demo_gcn.py feeds them (tf.SparseTensor, gcn.py:269-272): the pattern is fixed,
@@ -463,6 +472,7 @@ def build_workload(args, tfg, device):
         l1.build_cache_for_graph(graph)
         step = lambda xd: (l2([l1([pattern.with_value(xd), graph.edge_index, graph.edge_weight], cache=graph.cache),     # noqa: E731
                                graph.edge_index, graph.edge_weight], cache=graph.cache),)
+        outputs = ("gcn2",)
         nnz = int(x_host.numel())
         kernels["gcn_spmm"] = ("tfgk_spmm_f32", spmm_bytes(16, e_loop, True) + spmm_bytes(7, e_loop, True)
                                + nnz * (4 * 16 + 8) + n * (4 * 16 + 8),
@@ -479,6 +489,7 @@ def build_workload(args, tfg, device):
             loss = (out * g).sum()
             loss.backward()
             return (loss.detach().reshape(1), xg.grad)
+        outputs = ("loss", "x_grad")
         # forward mean aggregation (unweighted) + backward aggregation on the transposed CSR (weights 1/deg)
         kernels["sage_spmm"] = ("tfgk_spmm_f32", spmm_bytes(F, E, False) + spmm_bytes(F, E, True),
                                 "spmm kernels at D=100, forward + transposed backward (tfgk_spmm_f32)", None)
@@ -486,7 +497,26 @@ def build_workload(args, tfg, device):
         passes = 1
     else:
         raise ValueError(kind)
-    return {"x_host": x_host, "x": x, "step": step, "E": E, "n": n, "passes": passes, "kernels": kernels, "graph": graph}
+    return {"x_host": x_host, "x": x, "step": step, "outputs": outputs, "E": E, "n": n, "passes": passes, "kernels": kernels,
+            "graph": graph}
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(directory, names, outputs):
+    """Writes each output of one step as <directory>/<name>.npy in float32.  An output whose data exceeds its equal share
+    of DUMP_BYTES (less room for the .npy header) is stored as a fixed sample of its rows: the sorted result of
+    np.random.RandomState(0).choice(rows, k, replace=False), the same rows for every build at the same arguments."""
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // len(outputs) - 4096
+    for name, out in zip(names, outputs):
+        out = out.detach()
+        keep = share // (out[0].numel() * 4)
+        if keep < out.shape[0]:
+            rows = np.sort(np.random.RandomState(0).choice(out.shape[0], keep, replace=False))
+            out = out[torch.from_numpy(rows).to(out.device)]
+        np.save(os.path.join(directory, name + ".npy"), out.to(torch.float32).cpu().numpy())
 
 
 def run_ours(args, rank, world, local_rank):
@@ -496,6 +526,8 @@ def run_ours(args, rank, world, local_rank):
     device = torch.device("cuda", local_rank)
     torch.cuda.set_device(device)
     cfg = CONFIGS[args.config]
+    if args.dump_outputs and (world > 1 or cfg["kind"] == "gcn_partitioned"):
+        raise SystemExit("--dump-outputs is implemented for the single-GPU configs only")
     if world > 1 or cfg["kind"] == "gcn_partitioned":
         os.environ.setdefault("NCCL_DEBUG", "WARN")     # keep NCCL's version banner off stdout: one JSON line only
         import torch.distributed as dist
@@ -531,11 +563,15 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize()
     ev[0].record()
     for _ in range(args.steps):
-        step(x)
+        outputs = None            # the previous step's outputs are freed before the next step allocates, as when discarded
+        outputs = step(x)
     ev[1].record()
     torch.cuda.synchronize()
     clocks = sampler.stop()
     _ffi.set_trace(None)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wl["outputs"], outputs)
+    del outputs
     ms_step = ev[0].elapsed_time(ev[1]) / args.steps
     value = wl["passes"] * E / (ms_step * 1e-3)
 
@@ -625,6 +661,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     with StdoutToStderr():
         if args.impl == "reference":
+            if args.dump_outputs:
+                raise SystemExit("--dump-outputs writes the outputs of --impl ours")
             run_reference(args, rank, world)
         else:
             if not torch.cuda.is_available():

@@ -7,6 +7,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REQUIRED = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
             "dtype", "data", "config", "impl", "cpu_baseline", "e2e")
@@ -65,3 +67,41 @@ def test_gpu_arm_refuses_to_run_without_a_gpu():
     out = subprocess.run([sys.executable, "bench.py", "--steps", "1", "--warmup", "1"], cwd=ROOT, capture_output=True,
                          text=True, timeout=300)
     assert out.returncode != 0 and out.stdout.strip() == "" and "no CPU fallback" in out.stderr
+
+
+def test_dump_outputs_samples_large_outputs_to_a_fixed_row_set(tmp_path):
+    """Outputs above their share of 64 MB are stored as the same sorted row sample on every call; small ones whole."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    big = torch.arange(200000, dtype=torch.float32)[:, None].repeat(1, 128)      # each row holds its own index
+    small = torch.randn(1000, 16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ("big", "small"), (big, small))
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 * 1000 * 1000
+    got = np.load(tmp_path / "a" / "big.npy")
+    assert got.dtype == np.float32 and got.shape[1] == 128 and 0 < got.shape[0] < 200000
+    rows = got[:, 0].astype(np.int64)
+    assert np.all(np.diff(rows) > 0) and np.array_equal(got, big.numpy()[rows])
+    assert np.array_equal(got, np.load(tmp_path / "b" / "big.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small.numpy())
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_outputs_of_its_last_step(tmp_path):
+    """--dump-outputs on the headline step: one float32 file per layer, within 64 MB, the same arrays on a second run."""
+    import numpy as np
+    dumps = []
+    for run in ("first", "second"):
+        out = subprocess.run([sys.executable, "bench.py", "--steps", "2", "--warmup", "1", "--scale", "0.1", "--no-cpu-baseline",
+                              "--no-e2e", "--dump-outputs", str(tmp_path / run)], cwd=ROOT, capture_output=True, text=True,
+                             timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout)["steps"] == 2
+        assert sorted(os.listdir(tmp_path / run)) == ["gat.npy", "gcn.npy"]
+        assert sum(os.path.getsize(tmp_path / run / f) for f in os.listdir(tmp_path / run)) <= 64 * 1000 * 1000
+        dumps.append({f: np.load(tmp_path / run / f) for f in ("gat.npy", "gcn.npy")})
+    for f, a in dumps[0].items():
+        assert a.dtype == np.float32 and a.shape[1] == 128 and np.all(np.isfinite(a)) and np.any(a != 0), f
+        assert np.array_equal(a, dumps[1][f]), f
