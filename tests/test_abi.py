@@ -80,3 +80,13 @@ def test_product_never_imports_the_oracle():
                 assert "oracle" not in text.lower() or f in ("index_ops.cu", "__init__.py") and "import" not in \
                     [l for l in text.lower().splitlines() if "oracle" in l][0], \
                     "{} mentions the oracle".format(os.path.join(dirpath, f))
+
+
+def test_kernel_library_reads_no_environment_variable():
+    """Which kernel runs is decided from what the call can observe (shape, alignment, buffer layout), never from the
+    environment: a user-set variable must not change results or speed."""
+    csrc = os.path.join(ROOT, "tf_geometric_b200", "csrc")
+    for f in sorted(os.listdir(csrc)):
+        if f.endswith((".cu", ".cuh", ".h")):
+            text = open(os.path.join(csrc, f)).read()
+            assert "getenv" not in text, "{} reads an environment variable".format(f)

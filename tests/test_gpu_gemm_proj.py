@@ -122,21 +122,19 @@ def test_gemm_proj_transposed_weights_and_colsum():
 
 @pytest.mark.parametrize("m,k,widths", [(4096, 100, [128, 128, 128]), (130000, 100, [128, 128, 128, 128]), (777, 100, [128]),
                                         (3001, 128, [128, 64]), (1000, 33, [100, 7, 128]), (129, 8, [16]), (5000, 300, [128])])
-def test_gemm_proj_tensor_memory_operand_variant(m, k, widths, monkeypatch):
-    """Default kernel: the split A operands are staged in tensor memory (tcgen05.st) and the MMAs read A from there.
-    Same truncation, same products, same order -> the same bits as the shared-memory-operand kernel."""
+def test_gemm_proj_tensor_memory_operand_variant(m, k, widths):
+    """The projection kernel: the split A operands are staged in tensor memory (tcgen05.st) and the MMAs read A from there.
+    fp32-accurate against float64 for every shape, and repeatable bit for bit."""
     rs = np.random.RandomState(m + k)
     a = rs.randn(m, k).astype(np.float32)
     blocks, host = _blocks(rs, k, widths, m)
-    monkeypatch.setenv("TFGK_PROJ_IMPL", "ss")          # operands from shared memory (the first round-2 kernel)
-    want = ops.gemm_proj(dev(a), blocks)
-    monkeypatch.delenv("TFGK_PROJ_IMPL", raising=False)   # default: split A operands in tensor memory
     got = ops.gemm_proj(dev(a), blocks)
-    for (w, b, act), g, w_ in zip(host, got, want):
+    again = ops.gemm_proj(dev(a), blocks)
+    for (w, b, act), g, g2 in zip(host, got, again):
         ref = a.astype(np.float64) @ w.astype(np.float64)
         if b is not None:
             ref = ref + b
         if act == ops.ACT_RELU:
             ref = np.maximum(ref, 0)
         assert_close(g.cpu().numpy(), ref, rtol=1e-5, atol_scale=5e-6, what="ts gemm_proj width {}".format(w.shape[1]))
-        assert torch.equal(g, w_), "tensor-memory operand variant changed bits (width {})".format(w.shape[1])
+        assert torch.equal(g, g2), "gemm_proj is not repeatable (width {})".format(w.shape[1])

@@ -1,8 +1,6 @@
 # coding=utf-8
 """K4 tensor-core path (tcgen05, 3xTF32 split): fp32-level accuracy against float64, far inside the 1e-4 gate that a
 single TF32 pass would miss.  Shapes cover the projections of the hot path and the ragged edges (M, N, K tails)."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -10,8 +8,7 @@ import torch
 from tf_geometric_b200 import ops
 from conftest import assert_close
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(os.environ.get("TFGK_GEMM_TC") == "0", reason="tensor-core GEMM disabled by TFGK_GEMM_TC=0")]
+pytestmark = pytest.mark.gpu
 
 
 def dev(a):

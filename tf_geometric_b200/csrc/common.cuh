@@ -62,6 +62,34 @@ inline cudaError_t ensure_dynamic_smem(Kernel kernel, size_t bytes) {
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+struct alignas(64) TensorMap { uint64_t opaque[16]; };      // CUtensorMap (128 bytes), filled by the driver on the host
+
+// Encodes a 2-D fp32 tensor map over n_rows rows of `width` columns (row stride ld floats) whose box is one row: the
+// operand of TMA tile::gather4.  cuTensorMapEncodeTiled is reached through the runtime's driver entry point (no link-time
+// dependency on libcuda).  Returns TFGK_ERR_UNSUPPORTED when the driver cannot encode the map, so callers fall back.
+inline int make_row_tensor_map(TensorMap *out, const float *base, int64_t ld, int64_t n_rows, int32_t width) {
+    typedef int (*EncodeTiledFn)(void *map, int dtype, uint32_t rank, void *base, const uint64_t *dims,
+                                 const uint64_t *strides, const uint32_t *box, const uint32_t *elem_strides, int interleave,
+                                 int swizzle, int l2promo, int oob_fill);
+    static EncodeTiledFn encode = nullptr;
+    if (encode == nullptr) {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        TFGK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+        if (fn == nullptr || qres != cudaDriverEntryPointSuccess)
+            return set_error(TFGK_ERR_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
+        encode = reinterpret_cast<EncodeTiledFn>(fn);
+    }
+    const uint64_t dims[2] = {(uint64_t)width, (uint64_t)n_rows};
+    const uint64_t strides[1] = {(uint64_t)ld * sizeof(float)};           // byte stride of dimension 1 (rows)
+    const uint32_t box[2] = {(uint32_t)width, 1u};                        // gather4: 1 in the gathered dimension
+    const uint32_t elem[2] = {1u, 1u};
+    // CU_TENSOR_MAP_DATA_TYPE_FLOAT32 = 7, INTERLEAVE_NONE = 0, SWIZZLE_NONE = 0, L2_PROMOTION_L2_128B = 2, OOB_FILL_NONE = 0
+    const int rc = encode(out, 7, 2, const_cast<float *>(base), dims, strides, box, elem, 0, 0, 2, 0);
+    if (rc != 0) return set_error(TFGK_ERR_UNSUPPORTED, "cuTensorMapEncodeTiled failed with CUresult %d", rc);
+    return TFGK_OK;
+}
+
 // activation applied in every fused epilogue
 __device__ __forceinline__ float apply_act(float v, int act) {
     return act == TFGK_ACT_RELU ? fmaxf(v, 0.0f) : v;

@@ -10,8 +10,6 @@
 // roofline of the reference's 5-pass segment_softmax + two [E,A] gathers + SpMM pipeline (SURVEY.md 8d).
 // No tensor cores: the per-edge dot products are 16-wide and the kernel is bound by the gathers.
 #include "common.cuh"
-#include <stdlib.h>
-#include <string.h>
 
 namespace tfgk {
 
@@ -474,8 +472,6 @@ __global__ void __launch_bounds__(kGatAsyncWarps * 32) gat_async_kernel(const Ga
 // row lets ONE cp.async.bulk.tensor...tile::gather4 fetch the key AND the value rows of four neighbours (4 x 2A x 4 bytes = 4 KB
 // at A = 128) into the warp's ring stage, completing its mbarrier with the transaction bytes.  Arithmetic, edge order and the
 // online softmax are those of gat_async_kernel: same bits.  Requires V == K + A columns in the same buffer (ldk == ldv).
-struct alignas(64) GatTensorMap { uint64_t opaque[16]; };
-
 __device__ __forceinline__ void gat_mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;
     for (uint32_t spin = 0; !done; ++spin) {
@@ -489,7 +485,7 @@ __device__ __forceinline__ void gat_mbar_wait(uint32_t bar, uint32_t parity) {
 }
 
 template <int S>
-__global__ void __launch_bounds__(kGatAsyncWarps * 32) gat_gather4_kernel(const GatParams p, const __grid_constant__ GatTensorMap tmap) {
+__global__ void __launch_bounds__(kGatAsyncWarps * 32) gat_gather4_kernel(const GatParams p, const __grid_constant__ TensorMap tmap) {
     constexpr int U = 4, RPC = 32 / U;
     static_assert(S <= RPC, "index chunk refill assumes the prologue stays inside chunk 0");
     extern __shared__ __align__(128) uint8_t gat_g4_ring[];
@@ -694,28 +690,13 @@ static int launch_gat_async(const GatParams &p, cudaStream_t st) {
     return TFGK_OK;
 }
 
-typedef int (*GatEncodeTiledFn)(void *map, int dtype, uint32_t rank, void *base, const uint64_t *dims, const uint64_t *strides,
-                                const uint32_t *box, const uint32_t *elem_strides, int interleave, int swizzle, int l2promo,
-                                int oob_fill);
-
 template <int S>
 static int launch_gat_gather4(const GatParams &p, cudaStream_t st) {
     const int A = p.H * p.dqk;
     if (p.V != p.K + A || p.ldk != p.ldv || 2 * A > 256 || (p.ldk % 4) != 0) return TFGK_ERR_UNSUPPORTED;
-    static GatEncodeTiledFn encode = nullptr;
-    if (encode == nullptr) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        TFGK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (fn == nullptr || qres != cudaDriverEntryPointSuccess) return TFGK_ERR_UNSUPPORTED;
-        encode = reinterpret_cast<GatEncodeTiledFn>(fn);
-    }
-    GatTensorMap tmap;
-    const uint64_t dims[2] = {(uint64_t)(2 * A), (uint64_t)1 << 31};      // rows are bounded by the int32 column ids
-    const uint64_t strides[1] = {(uint64_t)p.ldk * sizeof(float)};
-    const uint32_t box[2] = {(uint32_t)(2 * A), 1u};
-    const uint32_t elem[2] = {1u, 1u};
-    if (encode(&tmap, 7, 2, const_cast<float *>(p.K), dims, strides, box, elem, 0, 0, 2, 0) != 0) return TFGK_ERR_UNSUPPORTED;
+    TensorMap tmap;
+    const int rc = make_row_tensor_map(&tmap, p.K, p.ldk, (int64_t)1 << 31, 2 * A);      // rows bounded by the int32 column ids
+    if (rc != TFGK_OK) return rc;
     const size_t stage_pitch = ((size_t)4 * 2 * A * 4 + 127) & ~(size_t)127;
     const size_t smem = (size_t)kGatAsyncWarps * S * stage_pitch + (size_t)kGatAsyncWarps * S * 8;
     TFGK_CUDA(ensure_dynamic_smem(gat_gather4_kernel<S>, smem));
@@ -731,23 +712,12 @@ static int launch_gat_gather4(const GatParams &p, cudaStream_t st) {
 }
 
 static int dispatch_gat_async(const GatParams &p, cudaStream_t st) {
-    // default: TMA tile::gather4 ring with two stages whenever K and V sit side by side in one buffer (the layers project them
-    // that way): 18.74 ms against 19.97 ms for the cp.async ring at the products shape, three / four stages lose resident warps
-    // (22.1 / 26.3 ms; profiles/r2_kernel_variants_final.json).  TFGK_GAT_IMPL=async keeps the cp.async ring; "gather4:S" sets S.
-    const char *g4 = getenv("TFGK_GAT_IMPL");
-    if (!(g4 && g4[0] == 'a')) {
-        const char *colon = g4 ? strchr(g4, ':') : nullptr;
-        const int stages = colon ? atoi(colon + 1) : 2;
-        const int rc = stages == 2 ? launch_gat_gather4<2>(p, st) : stages == 4 ? launch_gat_gather4<4>(p, st)
-                                                                              : launch_gat_gather4<3>(p, st);
-        if (rc != TFGK_ERR_UNSUPPORTED) return rc;
-    }
-    const char *cfg = getenv("TFGK_GAT_ASYNC_CFG");        // "UxS"; default 2x3
-    if (cfg && cfg[0] == '4' && cfg[2] == '2') return launch_gat_async<4, 2>(p, st);
-    if (cfg && cfg[0] == '4' && cfg[2] == '3') return launch_gat_async<4, 3>(p, st);
-    if (cfg && cfg[0] == '2' && cfg[2] == '4') return launch_gat_async<2, 4>(p, st);
-    if (cfg && cfg[0] == '2' && cfg[2] == '2') return launch_gat_async<2, 2>(p, st);
-    if (cfg && cfg[0] == '1' && cfg[2] == '4') return launch_gat_async<1, 4>(p, st);
+    // TMA tile::gather4 ring with two stages whenever K and V sit side by side in one buffer (the layers project them that
+    // way): 18.74 ms against 19.97 ms for the cp.async ring at the products shape on a B200, three / four stages lose resident
+    // warps (22.1 / 26.3 ms; profiles/r2_kernel_variants_final.json).  Separate K and V buffers, or a tensor map the driver
+    // cannot encode, take the cp.async ring.
+    const int rc = launch_gat_gather4<2>(p, st);
+    if (rc != TFGK_ERR_UNSUPPORTED) return rc;
     return launch_gat_async<2, 3>(p, st);
 }
 
@@ -949,11 +919,9 @@ static int gat_fused_impl(const int64_t *rowptr, const int32_t *col,
                       dqk <= 128 && dv % 4 == 0 && A <= 512 && VW <= 512 && ldq % 4 == 0 && ldk % 4 == 0 &&
                       ldv % 4 == 0 && ldo % 4 == 0 && aligned16(Q) && aligned16(K) && aligned16(V) && aligned16(out) &&
                       (!bias || aligned16(bias));
-    const char *impl = getenv("TFGK_GAT_IMPL");          // "twopass" forces the reference-order kernel
-    if (fast && dqk == dv && A <= 128 && !write_att && (stats != nullptr || !(impl && (impl[0] == 't' || impl[0] == 'o'))))
-        return dispatch_gat_async(p, st);                    // "online" forces the register-staged single-pass kernel
+    if (fast && dqk == dv && A <= 128 && !write_att) return dispatch_gat_async(p, st);
     if (stats != nullptr) return TFGK_ERR_UNSUPPORTED;      // only the streaming kernel keeps (max, denominator)
-    if (fast && dqk == dv && !(impl && impl[0] == 't')) {
+    if (fast && dqk == dv) {
         switch ((A + 127) / 128) {
             case 1: return launch_gat_online<1>(p, st);
             case 2: return launch_gat_online<2>(p, st);

@@ -235,9 +235,7 @@ extern "C" int tfgk_gemm_f32(const float *A, int64_t lda, int transA, const floa
     if (!transA && beta == 0.0f && K > 0) {
         // tall projections (and dX = dY W^T with transB): the multi-block tcgen05 kernel (gemm_proj.cu), N cut into blocks
         // of <= 128 columns
-        const char *env = getenv("TFGK_GEMM_TC");
-        const bool tc_on = !(env != nullptr && env[0] == '0');
-        if (tc_on && N <= 512 && (int64_t)M * K >= (1 << 14)) {
+        if (N <= 512 && (int64_t)M * K >= (1 << 14)) {
             tfgk_proj_block blocks[4];
             int nb = 0;
             for (int c0 = 0; c0 < N; c0 += 128, ++nb) {

@@ -17,7 +17,6 @@
 //     `first_part` so that every rank pulls from a different peer at any moment.
 #include "common.cuh"
 #include "tfgk_tc.cuh"
-#include <stdlib.h>
 
 namespace tfgk {
 namespace proj {
@@ -43,26 +42,9 @@ struct Params {
     int64_t lda, part_rows;
     int n_parts, first_tile, local_part;
     int M, K, nb, tiles_m, n_groups;
-    int dbg;           // measurement switches (TFGK_PROJ_DEBUG): 1 no lo conversion, 2 hi*hi MMA only, 4 no stores, 8 no loads,
-                       // 16 no TMEM reads, 32 no staging / stores after the TMEM read, 64 epilogue stores straight from registers
     const float *B[kMaxBlocks]; int64_t ldb[kMaxBlocks];
     const float *bias[kMaxBlocks]; int act[kMaxBlocks]; int ncols[kMaxBlocks]; int transb[kMaxBlocks];
     float *C[kMaxBlocks]; int64_t ldc[kMaxBlocks];
-};
-
-struct Plan {
-    uint32_t kpad8, b_bytes, a_stage_bytes, stages, total;
-    __host__ __device__ explicit Plan(int K) {
-        kpad8 = (uint32_t)((K + 7) / 8) * 8;
-        b_bytes = (uint32_t)kUN * kpad8 * 4u;
-        a_stage_bytes = 2u * BM * BK * 4u;
-        const uint32_t fixed = 2u * b_bytes + kEpilogueWarps * kStageBytes + kBarrierBytes + kUN * 4u;
-        const uint32_t budget = 227u * 1024u;
-        stages = 0;
-        for (uint32_t st = 4; st >= 2; --st)
-            if (fixed + st * a_stage_bytes <= budget) { stages = st; break; }
-        total = fixed + stages * a_stage_bytes;
-    }
 };
 
 __device__ __forceinline__ bool elect_one() {
@@ -71,7 +53,7 @@ __device__ __forceinline__ bool elect_one() {
     return pred != 0;
 }
 
-// ---- epilogue shared by both kernels: TMEM -> registers -> per-warp staging tile -> full row segments per store ----------
+// ---- epilogue: TMEM -> registers -> per-warp staging tile -> full row segments per store ------------------------------------
 __device__ __forceinline__ int tile_index(const Params &p, int group, int it) {
     int tl = group + it * p.n_groups + p.first_tile;
     return tl >= p.tiles_m ? tl - p.tiles_m : tl;
@@ -103,65 +85,10 @@ __device__ __forceinline__ void epilogue_loop(const Params &p, int cb, int group
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&acc_empty[buf]);
             }
-            if (p.dbg & 64) {
-                // direct variant: every thread stores the 16 columns of its own row straight from registers (64 contiguous
-                // bytes per row in four 16-byte stores), the tensor-memory read of the next pass is issued before the stores
-                // of this one - no staging tile, no warp barriers on the path
-                uint32_t ra[16], rb[16];
-                auto ldtm = [&](int ps, uint32_t (&r)[16]) {
-                    const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * kUN + ps * kPassCols);
-                    asm volatile(
-                        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                          "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                        : "r"(taddr));
-                };
-                auto store = [&](int ps, const uint32_t (&r)[16]) {
-                    const int c0 = ps * kPassCols;
-                    const int64_t row = row0 + lane;
-                    if (row >= p.M || (p.dbg & 4)) return;
-                    float *dst = Cb + row * ldc + c0;
-#pragma unroll
-                    for (int j = 0; j < 16; j += 4) {
-                        float4 v;
-                        v.x = apply_act(__uint_as_float(r[j]) + s_bias[c0 + j], act);
-                        v.y = apply_act(__uint_as_float(r[j + 1]) + s_bias[c0 + j + 1], act);
-                        v.z = apply_act(__uint_as_float(r[j + 2]) + s_bias[c0 + j + 2], act);
-                        v.w = apply_act(__uint_as_float(r[j + 3]) + s_bias[c0 + j + 3], act);
-                        if (vec_ok && c0 + j + 4 <= ncols) {
-                            *reinterpret_cast<float4 *>(dst + j) = v;
-                        } else {
-                            if (c0 + j < ncols) dst[j] = v.x;
-                            if (c0 + j + 1 < ncols) dst[j + 1] = v.y;
-                            if (c0 + j + 2 < ncols) dst[j + 2] = v.z;
-                            if (c0 + j + 3 < ncols) dst[j + 3] = v.w;
-                        }
-                    }
-                };
-                if (pass0 < pass1) ldtm(pass0, ra);
-                for (int ps = pass0; ps < pass1; ps += 2) {
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (ps + 1 < pass1) ldtm(ps + 1, rb);
-                    else { tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive(&acc_empty[buf]); }
-                    store(ps, ra);
-                    if (ps + 1 < pass1) {
-                        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                        if (ps + 2 < pass1) ldtm(ps + 2, ra);
-                        else { tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive(&acc_empty[buf]); }
-                        store(ps + 1, rb);
-                    }
-                }
-                continue;
-            }
             for (int ps = pass0; ps < pass1; ++ps) {
                 const int c0 = ps * kPassCols;
                 uint32_t r[16];
                 const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * kUN + c0);
-                if (p.dbg & 16) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) r[j] = 0;
-                } else
                 asm volatile(
                     "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
                     "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
@@ -174,7 +101,6 @@ __device__ __forceinline__ void epilogue_loop(const Params &p, int cb, int group
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&acc_empty[buf]);
                 }
-                if (p.dbg & 32) continue;
 #pragma unroll
                 for (int j = 0; j < 16; j += 4) {
                     const float v0 = apply_act(__uint_as_float(r[j]) + s_bias[c0 + j], act);
@@ -190,7 +116,7 @@ __device__ __forceinline__ void epilogue_loop(const Params &p, int cb, int group
                     const int rl = j * 8 + seg_row;
                     const int64_t row = row0 + rl;
                     const float4 v = *reinterpret_cast<const float4 *>(stg + rl * kStageRowBytes + seg_chunk * 16);
-                    if (row < p.M && !(p.dbg & 4)) {
+                    if (row < p.M) {
                         float *dst = Cb + row * ldc + col;
                         if (vec_ok && col + 4 <= ncols) {
                             *reinterpret_cast<float4 *>(dst) = v;
@@ -207,189 +133,8 @@ __device__ __forceinline__ void epilogue_loop(const Params &p, int cb, int group
         }
 }
 
-template <int STAGES>
-__global__ void __launch_bounds__(kThreadsProj, 1) gemm_proj_kernel(const Params p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const Plan L(p.K);
-    uint8_t *b_hi_ptr = smem, *b_lo_ptr = smem + L.b_bytes;
-    uint8_t *a_ring = smem + 2 * L.b_bytes;
-    uint8_t *stage_base = a_ring + STAGES * L.a_stage_bytes;
-    uint64_t *full = reinterpret_cast<uint64_t *>(stage_base + kEpilogueWarps * kStageBytes);
-    uint64_t *empty = full + STAGES, *landed = empty + STAGES, *acc_full = landed + STAGES, *acc_empty = acc_full + 2;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(acc_empty + 2);
-    float *s_bias = reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(full) + kBarrierBytes);
-    const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-    const int cb = (int)blockIdx.x % p.nb, group = (int)blockIdx.x / p.nb;
-    const int ncols = p.ncols[cb];
-    const int un = ((ncols + 15) / 16) * 16;
-    const float *__restrict__ Bm = p.B[cb];
-    const int64_t ldb = p.ldb[cb];
-    const bool tb = p.transb[cb] != 0;
-
-    for (int i = t; i < kUN; i += kThreadsProj) s_bias[i] = (p.bias[cb] != nullptr && i < ncols) ? __ldg(p.bias[cb] + i) : 0.0f;
-    if (t == 0) {
-        for (int i = 0; i < STAGES; ++i) {
-            mbar_init(&full[i], kProducerWarps); mbar_init(&empty[i], 1); mbar_init(&landed[i], kLoaderWarps * 32);
-        }
-        for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], kEpilogueWarps); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemColsProj) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    {   // W_b: transpose + RNA split into the K-major core-matrix layout, once per CTA
-        const int kchunks = (int)L.kpad8 / 4;
-        const int total = un * kchunks;
-        const uint32_t bh = smem_u32(b_hi_ptr), bl = smem_u32(b_lo_ptr);
-        for (int c = t; c < total; c += kThreadsProj) {
-            const int n8 = c & 7, kc = (c >> 3) % kchunks, ng = (c >> 3) / kchunks;
-            const int n = ng * 8 + n8, k = kc * 4;
-            float w[4] = {0.f, 0.f, 0.f, 0.f}, h[4], l[4];
-            if (n < ncols) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    if (k + i < p.K) w[i] = __ldg(tb ? Bm + (int64_t)n * ldb + (k + i) : Bm + (int64_t)(k + i) * ldb + n);
-            }
-#pragma unroll
-            for (int i = 0; i < 4; ++i) split_tf32(w[i], h[i], l[i]);
-            st_shared_v4(bh + c * 16, h[0], h[1], h[2], h[3]);
-            st_shared_v4(bl + c * 16, l[0], l[1], l[2], l[3]);
-        }
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const int nkb = (int)(L.kpad8 + BK - 1) / BK;
-    const int last_steps = ((int)L.kpad8 - (nkb - 1) * BK) / UMMA_K;
-    const int my_tiles = group < p.tiles_m ? (p.tiles_m - 1 - group) / p.n_groups + 1 : 0;
-    const int total_kb = my_tiles * nkb;
-    // logical tile i of this group -> physical row tile (rotated so that ranks start on different parts)
-    auto tile_of = [&](int it) {
-        int tl = group + it * p.n_groups + p.first_tile;
-        return tl >= p.tiles_m ? tl - p.tiles_m : tl;
-    };
-
-    if (warp >= kLoaderWarp0) {
-        // ===================== loaders: cp.async A (possibly from a peer GPU) straight into the UMMA layout =====================
-        // The round-1 kernel (and the first version of this one) let the same threads load AND convert: a k-block could only be
-        // published after the thread had blocked on the stage for a later load, so producer, tensor core and the commit
-        // round trip (~1000 cycles, measured with the TFGK_PROJ_DEBUG switches) ran one after the other.  Here every
-        // role blocks only on its own dependency: loaders on `empty`, converters on `landed`, the MMA issuer on `full`.
-        const int tl = t - kLoaderWarp0 * 32;                                // 0..63
-        const uint32_t a_ring_addr = smem_u32(a_ring);
-        constexpr int kChunks = (BM * BK / 4) / (kLoaderWarps * 32);        // 16 per thread per k-block
-        const int r8 = tl & 7, kc = (tl >> 3) & 7;                          // chunk c = tl + 64 i: rows i * 8 + r8
-        // L2 prefetch of whole row tiles kPrefetchTiles ahead (one bulk-prefetch instruction per tile, issued by the group's
-        // first column block).  Peer-mapped parts are not prefetched (remote data bypasses the local L2).
-        constexpr int kPrefetchTiles = 4;
-        const bool can_prefetch = (cb == 0) && (tl == 0) && p.lda <= 2 * (int64_t)p.K;
-        auto prefetch_tile = [&](int it) {
-            if (!can_prefetch || it >= my_tiles) return;
-            const int64_t m0 = (int64_t)tile_of(it) * BM;
-            const int part = p.n_parts > 1 ? (int)(m0 / p.part_rows) : 0;
-            if (p.n_parts > 1 && part != p.local_part) return;
-            const int64_t rows = min((int64_t)BM, (int64_t)p.M - m0);
-            const float *src = p.A[part] + (m0 - (int64_t)part * p.part_rows) * p.lda;
-            const uint32_t bytes = (uint32_t)(rows * p.lda * 4);
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-        };
-        for (int i = 0; i < kPrefetchTiles; ++i) prefetch_tile(i);
-        for (int G = 0; G < total_kb; ++G) {
-            const int stage = G % STAGES;
-            mbar_wait(&empty[stage], (uint32_t)(((G / STAGES) & 1) ^ 1));      // MMAs of k-block G - STAGES retired
-            const int tile = tile_of(G / nkb), kb = G % nkb;
-            if (kb == 0) prefetch_tile(G / nkb + kPrefetchTiles);
-            const int k = kb * BK + kc * 4;
-            if (k < (int)L.kpad8 && !(p.dbg & 8)) {
-                const int64_t m0 = (int64_t)tile * BM;
-                const int part = p.n_parts > 1 ? (int)(m0 / p.part_rows) : 0;
-                const float *base = p.A[part] + (m0 - (int64_t)part * p.part_rows) * p.lda + k;
-                const uint32_t kbytes = k < p.K ? (uint32_t)min(4, p.K - k) * 4u : 0u;
-                const uint32_t dst0 = a_ring_addr + stage * L.a_stage_bytes + (uint32_t)tl * 16u;
-#pragma unroll
-                for (int i = 0; i < kChunks; ++i) {
-                    const int rl = i * 8 + r8;
-                    const bool ok = m0 + rl < p.M;
-                    cp_async16_zfill(dst0 + (uint32_t)i * 1024u, ok ? base + (int64_t)rl * p.lda : p.A[0], ok ? kbytes : 0u);
-                }
-            }
-            // the stage's `landed` barrier completes when the copies of all 64 loader threads have arrived
-            asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(&landed[stage])) : "memory");
-        }
-    } else if (warp < kProducerWarps) {
-        // ===================== converters: lo = a - trunc_tf32(a) for every landed k-block =====================
-        constexpr int kChunks = (BM * BK / 4) / (kProducerWarps * 32);      // 8 per thread per k-block
-        const int kc = (t >> 3) & 7;                                        // chunk c = t + 128 i
-        for (int G = 0; G < total_kb; ++G) {
-            const int stage = G % STAGES, kb = G % nkb;
-            mbar_wait(&landed[stage], (uint32_t)((G / STAGES) & 1));
-            if (kb * BK + kc * 4 < (int)L.kpad8 && !(p.dbg & 1)) {
-                uint8_t *sraw = a_ring + stage * L.a_stage_bytes + t * 16;
-#pragma unroll
-                for (int i = 0; i < kChunks; ++i) {
-                    const float4 v = *reinterpret_cast<const float4 *>(sraw + i * 2048);
-                    float4 l;
-                    l.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
-                    l.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
-                    l.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
-                    l.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
-                    *reinterpret_cast<float4 *>(sraw + BM * BK * 4 + i * 2048) = l;
-                }
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&full[stage]);
-        }
-    } else if (warp == kProducerWarps + kEpilogueWarps) {
-        // ===================== MMA issuer (warp-uniform loop, one elected lane issues; see the TS kernel) =====================
-        const uint32_t idesc = make_idesc(un);
-        const uint32_t sbo_b = (L.kpad8 / 4) * 128u;
-        const uint64_t dbh0 = make_desc_sbo(smem_u32(b_hi_ptr), sbo_b), dbl0 = make_desc_sbo(smem_u32(b_lo_ptr), sbo_b);
-        const uint32_t a_ring0 = smem_u32(a_ring);
-        int stage = 0, kb = 0, it = 0;
-        uint32_t stage_phase = 0;
-        for (int G = 0; G < total_kb; ++G) {
-            const int buf = it & 1;
-            if (kb == 0) mbar_wait(&acc_empty[buf], (uint32_t)(((it >> 1) & 1) ^ 1));
-            mbar_wait(&full[stage], stage_phase);
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(buf * kUN);
-            const uint32_t a_raw = a_ring0 + (uint32_t)stage * L.a_stage_bytes;
-            const uint64_t dah0 = make_desc_sbo(a_raw, 1024u), dal0 = make_desc_sbo(a_raw + BM * BK * 4, 1024u);
-            const uint64_t dbh = dbh0 + (uint64_t)(kb * 64), dbl = dbl0 + (uint64_t)(kb * 64);
-            const int steps = kb == nkb - 1 ? last_steps : BK / UMMA_K;
-            if (elect_one()) {
-#pragma unroll
-                for (int j = 0; j < BK / UMMA_K; ++j) {
-                    if (j < steps) {
-                        const uint64_t o = (uint64_t)(j * 16);
-                        if (p.dbg & 2) { umma_tf32(d_tmem, dah0 + o, dbh + o, idesc, (kb | j) != 0); continue; }
-                        umma_tf32(d_tmem, dal0 + o, dbh + o, idesc, (kb | j) != 0);
-                        umma_tf32(d_tmem, dah0 + o, dbl + o, idesc, 1u);
-                        umma_tf32(d_tmem, dah0 + o, dbh + o, idesc, 1u);
-                    }
-                }
-                umma_commit(&empty[stage]);
-                if (kb == nkb - 1) umma_commit(&acc_full[buf]);
-            }
-            __syncwarp();
-            if (++stage == STAGES) { stage = 0; stage_phase ^= 1u; }
-            if (++kb == nkb) { kb = 0; ++it; }
-        }
-    } else {
-        epilogue_loop(p, cb, group, un, ncols, tmem_base, stage_base, s_bias, acc_full, acc_empty, my_tiles, warp, lane);
-    }
-    __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemColsProj) : "memory");
-    }
-}
-
-// ---- variant with the A operands in tensor memory ("TS" form of tcgen05.mma) -----------------------------------------------
-// Measured on the kernel above (TFGK_PROJ_DEBUG switches, profiles/r2_notes.md): a ring stage makes one trip
+// ---- the kernel: A operands in tensor memory ("TS" form of tcgen05.mma) ----------------------------------------------------
+// Why tensor memory (profiles/r2_notes.md): with the split A operands in shared memory, a ring stage makes one trip
 // free -> load -> convert -> MMA -> commit -> free in ~3000 cycles whatever its size, and next to the resident W the ring
 // holds raw + lo tiles for only 96 K-columns - less than one 128 x 104 row tile - so a row tile costs about one full trip
 // (4.3 us) where its 39 MMAs need 1.3 us.  Here the ring in shared memory holds RAW k-blocks only (16 KB per 32 columns,
@@ -518,7 +263,7 @@ __global__ void __launch_bounds__(kThreadsProj, 1) gemm_proj_ts_kernel(const Par
             const int tile = tile_index(p, group, G / nkb), kb = G % nkb;
             if (kb == 0) prefetch_tile(G / nkb + kPrefetchTiles);
             const int k = kb * BK + kc * 4;
-            if (k < (int)L.kpad8 && !(p.dbg & 8)) {
+            if (k < (int)L.kpad8) {
                 const int64_t m0 = (int64_t)tile * BM;
                 const int part = p.n_parts > 1 ? (int)(m0 / p.part_rows) : 0;
                 const float *base = p.A[part] + (m0 - (int64_t)part * p.part_rows) * p.lda + k;
@@ -555,7 +300,7 @@ __global__ void __launch_bounds__(kThreadsProj, 1) gemm_proj_ts_kernel(const Par
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
                 float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (kb * BK + c * 4 < (int)L.kpad8 && !(p.dbg & 1)) v = *reinterpret_cast<const float4 *>(row + ((c ^ (t & 7)) * 16));
+                if (kb * BK + c * 4 < (int)L.kpad8) v = *reinterpret_cast<const float4 *>(row + ((c ^ (t & 7)) * 16));
                 const float a[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
@@ -601,7 +346,6 @@ __global__ void __launch_bounds__(kThreadsProj, 1) gemm_proj_ts_kernel(const Par
                     if (j < steps) {
                         const uint64_t bh = dbh + (uint64_t)(j * 16), bl = dbl + (uint64_t)(j * 16);           // + j * 256 bytes
                         const uint32_t ah = a_hi + (uint32_t)(j * UMMA_K), al = ah + 32u;
-                        if (p.dbg & 2) { umma_tf32_ts(d_tmem, ah, bh, idesc, (kb | j) != 0); continue; }
                         umma_tf32_ts(d_tmem, al, bh, idesc, (kb | j) != 0);
                         umma_tf32_ts(d_tmem, ah, bl, idesc, 1u);
                         umma_tf32_ts(d_tmem, ah, bh, idesc, 1u);
@@ -637,20 +381,6 @@ static int launch_ts(const Params &p, int grid, uint32_t smem_bytes, cudaStream_
     return TFGK_OK;
 }
 
-template <int STAGES>
-static int launch(const Params &p, int grid, uint32_t smem_bytes, cudaStream_t st) {
-    static int configured[16] = {0};       // cudaFuncSetAttribute once per device, not per call
-    int dev = 0;
-    TFGK_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 16 || configured[dev] < (int)smem_bytes) {
-        TFGK_CUDA(cudaFuncSetAttribute(gemm_proj_kernel<STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-        if (dev >= 0 && dev < 16) configured[dev] = (int)smem_bytes;
-    }
-    gemm_proj_kernel<STAGES><<<grid, kThreadsProj, smem_bytes, st>>>(p);
-    TFGK_LAUNCH_CHECK();
-    return TFGK_OK;
-}
-
 }  // namespace proj
 }  // namespace tfgk
 
@@ -677,7 +407,6 @@ extern "C" int tfgk_gemm_proj_f32(const float *const *A_parts, int32_t n_parts, 
     }
     p.lda = lda; p.part_rows = n_parts > 1 ? part_rows : (int64_t)1 << 40; p.n_parts = n_parts;
     p.M = M; p.K = K; p.nb = n_blocks;
-    { const char *d = getenv("TFGK_PROJ_DEBUG"); p.dbg = d ? atoi(d) : 0; }
     p.tiles_m = (int)ceil_div64(M, tc::BM);
     p.first_tile = n_parts > 1 ? (int)((int64_t)first_part * part_rows / tc::BM) : 0;
     p.local_part = n_parts > 1 ? (first_part + n_parts - 1) % n_parts : 0;      // the walk starts one past the caller's own part
@@ -695,8 +424,10 @@ extern "C" int tfgk_gemm_proj_f32(const float *const *A_parts, int32_t n_parts, 
         p.transb[b] = blk.transB;
         p.C[b] = blk.C; p.ldc[b] = blk.ldc;
     }
-    const proj::Plan L(K);
-    if (L.stages == 0) return TFGK_ERR_UNSUPPORTED;
+    // K <= 136, i.e. at least four raw stages next to the resident W: the range this kernel is tested and measured on.
+    // Wider K (up to 512) goes to gemm_tc.cu through tfgk_gemm_f32's fallback on TFGK_ERR_UNSUPPORTED.
+    const proj::PlanTS L(K);
+    if (L.stages < 4) return TFGK_ERR_UNSUPPORTED;
     int dev = 0, sms = 0;
     TFGK_CUDA(cudaGetDevice(&dev));
     TFGK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -707,20 +438,9 @@ extern "C" int tfgk_gemm_proj_f32(const float *const *A_parts, int32_t n_parts, 
     p.n_groups = n_groups;
     const int grid = n_groups * n_blocks;
     cudaStream_t st = as_stream(stream);
-    {   // A operands through tensor memory (TFGK_PROJ_IMPL=ss selects the all-shared-memory kernel)
-        const char *impl = getenv("TFGK_PROJ_IMPL");
-        const proj::PlanTS LT(K);
-        if (!(impl != nullptr && impl[0] == 's') && LT.stages >= 2) {
-            switch (LT.stages) {
-                case 6: return proj::launch_ts<6>(p, grid, LT.total, st);
-                case 5: return proj::launch_ts<5>(p, grid, LT.total, st);
-                case 4: return proj::launch_ts<4>(p, grid, LT.total, st);
-                case 3: return proj::launch_ts<3>(p, grid, LT.total, st);
-                default: return proj::launch_ts<2>(p, grid, LT.total, st);
-            }
-        }
+    switch (L.stages) {
+        case 6: return proj::launch_ts<6>(p, grid, L.total, st);
+        case 5: return proj::launch_ts<5>(p, grid, L.total, st);
+        default: return proj::launch_ts<4>(p, grid, L.total, st);
     }
-    if (L.stages >= 4) return proj::launch<4>(p, grid, L.total, st);
-    if (L.stages == 3) return proj::launch<3>(p, grid, L.total, st);
-    return proj::launch<2>(p, grid, L.total, st);
 }

@@ -1,5 +1,6 @@
-// K4 (tensor-core path): C[M,N] = act(A[M,K] @ B[K,N] + bias) for the dense projections x@W of the hot path
-// (nn/conv/gcn.py:272, gat.py:52,61,70, graph_sage.py:43-44, appnp.py:69) on the 5th-generation tensor cores.
+// K4 (tensor-core path for the projections gemm_proj.cu does not take): C[M,N] = act(A[M,K] @ B[K,N] + bias) with
+// 136 < K <= 512 and N <= 256, e.g. a 512-wide input projected to 16 columns.  tfgk_gemm_f32 tries tfgk_gemm_proj_f32
+// first and comes here when that returns TFGK_ERR_UNSUPPORTED (non-transposed B only); everything else is the SIMT kernel.
 //
 //   * tcgen05.mma.cta_group::1.kind::tf32, UMMA 128 x UN x 8, fp32 accumulators in TMEM (2 x UN columns, double buffered)
 //   * fp32-accurate via the 3xTF32 split: a = hi + lo with hi = rna_tf32(a), lo = a - hi (exact);
@@ -13,7 +14,6 @@
 // The kernel is memory bound (4(MK+MN) bytes for ~6MNK tf32 flops at K~100): the tensor pipe is lightly loaded by design.
 #include "common.cuh"
 #include "tfgk_tc.cuh"
-#include <stdlib.h>
 
 namespace tfgk {
 namespace tc {
@@ -39,179 +39,9 @@ struct SmemPlan {
     }
 };
 
-
-
-template <int STAGES>
-__global__ void __launch_bounds__(kThreads, 1) gemm_tf32x3_kernel(const Params p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const SmemPlan L(p.un, p.K);
-    uint8_t *b_hi_ptr = smem, *b_lo_ptr = smem + L.b_bytes;
-    uint8_t *a_ring = smem + 2 * L.b_bytes;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(a_ring + STAGES * L.a_stage_bytes);   // [STAGES] stage free, [2] acc full
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + STAGES + 2);
-    const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-
-    if (t == 0) {
-        for (int i = 0; i < STAGES + 2; ++i) mbar_init(&bars[i], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    // ---- W: transpose + RNA split, once per CTA ----
-    {
-        const int kchunks = (int)L.kpad / 4;
-        const int total = p.un * kchunks;
-        const uint32_t bh = smem_u32(b_hi_ptr), bl = smem_u32(b_lo_ptr);
-        for (int cb = t; cb < total; cb += kThreads) {
-            const int n8 = cb & 7, kc = (cb >> 3) % kchunks, ng = (cb >> 3) / kchunks;
-            const int n = ng * 8 + n8, k = kc * 4;
-            float w[4] = {0.f, 0.f, 0.f, 0.f}, h[4], l[4];
-            if (n < p.N) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    if (k + i < p.K) w[i] = __ldg(p.B + (int64_t)(k + i) * p.ldb + n);
-            }
-#pragma unroll
-            for (int i = 0; i < 4; ++i) split_tf32(w[i], h[i], l[i]);
-            st_shared_v4(bh + cb * 16, h[0], h[1], h[2], h[3]);
-            st_shared_v4(bl + cb * 16, l[0], l[1], l[2], l[3]);
-        }
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t idesc = make_idesc(p.un);
-    const int nkb = (int)L.kpad / BK;
-    const uint32_t sbo_b = (L.kpad / 4) * 128u;
-    const int my_tiles = blockIdx.x < p.tiles_m ? (p.tiles_m - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-    const int total_kb = my_tiles * nkb;
-    const uint32_t a_ring_addr = smem_u32(a_ring);
-
-    auto issue_load = [&](int G) {
-        if (G < total_kb) {
-            const int stage = G % STAGES;
-            if (G >= STAGES) mbar_wait(&bars[stage], (uint32_t)((G / STAGES - 1) & 1));   // MMAs that read this stage retired
-            const int tile = blockIdx.x + (G / nkb) * gridDim.x, kb = G % nkb;
-            const int64_t m0 = (int64_t)tile * BM;
-            const uint32_t dst0 = a_ring_addr + stage * L.a_stage_bytes;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int c = t + kThreads * i;
-                const int r8 = c & 7, kc = (c >> 3) & 7, rg = c >> 6;
-                const int64_t row = m0 + rg * 8 + r8;
-                const int k = kb * BK + kc * 4;
-                uint32_t bytes = 0;
-                const float *src = p.A;
-                if (row < p.M && k < p.K) {
-                    bytes = (uint32_t)min(4, p.K - k) * 4u;
-                    src = p.A + row * p.lda + k;
-                }
-                cp_async16_zfill(dst0 + c * 16, src, bytes);
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-
-    auto epilogue = [&](int tile, int buf, uint32_t use) {
-        mbar_wait(&bars[STAGES + buf], use & 1u);
-        tc_fence_after();
-        const int q = warp & 3, half = warp >> 2;
-        const int64_t row = (int64_t)tile * BM + q * 32 + lane;
-        const int col_begin = half * (p.un / 2), col_end = (half + 1) * (p.un / 2);
-        const bool vec_ok = (p.ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
-        for (int c0 = col_begin; c0 < col_end; c0 += 8) {
-            uint32_t r[8];
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * kMaxUN + c0);
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                         : "r"(taddr));
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            if (row < p.M) {
-                float v[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    v[j] = __uint_as_float(r[j]);
-                    if (p.bias && c0 + j < p.N) v[j] += __ldg(p.bias + c0 + j);
-                    v[j] = apply_act(v[j], p.act);
-                }
-                float *dst = p.C + row * p.ldc + c0;
-                if (vec_ok && c0 + 8 <= p.N) {
-                    *reinterpret_cast<float4 *>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-                    *reinterpret_cast<float4 *>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j)
-                        if (c0 + j < p.N) dst[j] = v[j];
-                }
-            }
-        }
-        tc_fence_before();
-    };
-
-#pragma unroll
-    for (int G = 0; G < STAGES - 1; ++G) issue_load(G);
-
-    int prev_tile = -1;
-    for (int G = 0; G < total_kb; ++G) {
-        issue_load(G + STAGES - 1);
-        asm volatile("cp.async.wait_group %0;" ::"n"(STAGES - 1) : "memory");
-        const int stage = G % STAGES;
-        const int it = G / nkb, kb = G % nkb;             // CTA-local tile counter, k-block within the tile
-        const int tile = blockIdx.x + it * gridDim.x;
-        const int buf = it & 1;
-        uint8_t *sraw = a_ring + stage * L.a_stage_bytes;
-        uint8_t *slo = sraw + BM * BK * 4;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {                       // lo = a - trunc_tf32(a), on the chunks this thread copied itself
-            const int c = t + kThreads * i;
-            const float4 v = *reinterpret_cast<const float4 *>(sraw + c * 16);
-            float4 l;
-            l.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
-            l.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
-            l.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
-            l.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
-            *reinterpret_cast<float4 *>(slo + c * 16) = l;
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        tc_fence_before();
-        __syncthreads();
-        if (t == 0) {
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(buf * kMaxUN);
-            const uint32_t a_raw = smem_u32(sraw), a_lo = a_raw + BM * BK * 4;
-            const uint32_t b_hi = smem_u32(b_hi_ptr) + (uint32_t)kb * (BK / 4) * 128u, b_lo = b_hi + L.b_bytes;
-#pragma unroll
-            for (int j = 0; j < BK / UMMA_K; ++j) {
-                const uint32_t off = (uint32_t)j * 2u * 128u;
-                const uint64_t dah = make_desc_sbo(a_raw + off, 1024u), dal = make_desc_sbo(a_lo + off, 1024u);
-                const uint64_t dbh = make_desc_sbo(b_hi + off, sbo_b), dbl = make_desc_sbo(b_lo + off, sbo_b);
-                umma_tf32(d_tmem, dal, dbh, idesc, (kb | j) != 0);
-                umma_tf32(d_tmem, dah, dbl, idesc, 1u);
-                umma_tf32(d_tmem, dah, dbh, idesc, 1u);
-            }
-            umma_commit(&bars[stage]);
-            if (kb == nkb - 1) umma_commit(&bars[STAGES + buf]);
-        }
-        if (kb == nkb - 1) {
-            if (prev_tile >= 0) epilogue(prev_tile, buf ^ 1, (uint32_t)((it - 1) >> 1));
-            prev_tile = tile;
-        }
-    }
-    if (prev_tile >= 0) epilogue(prev_tile, (my_tiles - 1) & 1, (uint32_t)((my_tiles - 1) >> 1));
-
-    __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-    }
-}
-
-// ---- warp-specialised variant -----------------------------------------------------------------------------------------
-// Same data path as gemm_tf32x3_kernel, but the three phases run concurrently in different warps and hand over through
-// mbarriers only (no __syncthreads in the steady state):
+// ---- warp-specialised kernel ------------------------------------------------------------------------------------------
+// The three phases run concurrently in different warps and hand over through mbarriers only (no __syncthreads in the
+// steady state):
 //   warps 0-3   producers : cp.async the next A k-block into the ring (after `empty[stage]`), convert lo for the k-block that
 //                           has landed (own chunks only), fence.proxy.async, one arrive per warp on `full[stage]`
 //   warps 4-11  epilogue  : wait `acc_full[buf]`, tcgen05.ld -> +bias -> act -> global, one arrive per warp on `acc_empty[buf]`
@@ -219,7 +49,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tf32x3_kernel(const Params p
 //                           tcgen05.commit -> `empty[stage]` (+ `acc_full[buf]` after the last k-block of the tile)
 constexpr int kWsProducerWarps = 4, kWsEpilogueWarps = 8;
 constexpr int kWsThreads = (kWsProducerWarps + kWsEpilogueWarps + 1) * 32;
-
 
 template <int STAGES>
 __global__ void __launch_bounds__(kWsThreads, 1) gemm_tf32x3_ws_kernel(const Params p) {
@@ -393,200 +222,6 @@ __global__ void __launch_bounds__(kWsThreads, 1) gemm_tf32x3_ws_kernel(const Par
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
     }
 }
-
-// ---- warp-specialised variant with a deep raw ring ------------------------------------------------------------------------
-// Little's law: the A stream needs ~60 KB in flight per SM; with raw and lo buffers tied together (32 KB per stage) only three
-// stages fit next to the resident W.  Here the cp.async ring holds RAW k-blocks only (16 KB each, R stages) while two lo buffers
-// alternate (lo[G % 2] is free again when the MMAs of k-block G-2 have retired - the same `empty` phase the raw stage of G-2
-// completes), W is stored for K rounded up to 8 instead of 32, and the MMA issuer skips the UMMA_K steps that lie beyond K.
-struct SmemPlanDeep {
-    uint32_t kpad_b, b_bytes, raw_bytes, ring, total;
-    __host__ __device__ SmemPlanDeep(int un, int K) {
-        kpad_b = (uint32_t)((K + 7) / 8) * 8;
-        b_bytes = (uint32_t)un * kpad_b * 4u;
-        raw_bytes = BM * BK * 4u;
-        const uint32_t budget = 227u * 1024u - 256u;
-        ring = 0;
-        for (uint32_t r = 5; r >= 3; --r)
-            if (2u * b_bytes + (r + 2u) * raw_bytes + 256u <= budget) { ring = r; break; }
-        total = 2u * b_bytes + (ring + 2u) * raw_bytes + 256u;
-    }
-};
-
-template <int R>
-__global__ void __launch_bounds__(kWsThreads, 1) gemm_tf32x3_deep_kernel(const Params p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const SmemPlanDeep L(p.un, p.K);
-    uint8_t *b_hi_ptr = smem, *b_lo_ptr = smem + L.b_bytes;
-    uint8_t *raw_ring = smem + 2 * L.b_bytes;                 // 1024-byte aligned: b_bytes is a multiple of 16*kpad_b*... see host check
-    uint8_t *lo_bufs = raw_ring + R * L.raw_bytes;
-    uint64_t *full = reinterpret_cast<uint64_t *>(lo_bufs + 2 * L.raw_bytes);
-    uint64_t *empty = full + R, *acc_full = empty + R, *acc_empty = acc_full + 2;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(acc_empty + 2);
-    const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-
-    if (t == 0) {
-        for (int i = 0; i < R; ++i) { mbar_init(&full[i], kWsProducerWarps); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], kWsEpilogueWarps); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    {
-        const int kchunks = (int)L.kpad_b / 4;
-        const int total = p.un * kchunks;
-        const uint32_t bh = smem_u32(b_hi_ptr), bl = smem_u32(b_lo_ptr);
-        for (int cb = t; cb < total; cb += kWsThreads) {
-            const int n8 = cb & 7, kc = (cb >> 3) % kchunks, ng = (cb >> 3) / kchunks;
-            const int n = ng * 8 + n8, k = kc * 4;
-            float w[4] = {0.f, 0.f, 0.f, 0.f}, h[4], l[4];
-            if (n < p.N) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    if (k + i < p.K) w[i] = __ldg(p.B + (int64_t)(k + i) * p.ldb + n);
-            }
-#pragma unroll
-            for (int i = 0; i < 4; ++i) split_tf32(w[i], h[i], l[i]);
-            st_shared_v4(bh + cb * 16, h[0], h[1], h[2], h[3]);
-            st_shared_v4(bl + cb * 16, l[0], l[1], l[2], l[3]);
-        }
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const int nkb = (p.K + BK - 1) / BK;
-    const int last_steps = ((p.K - (nkb - 1) * BK) + UMMA_K - 1) / UMMA_K;      // UMMA_K steps that hold real columns
-    const int my_tiles = blockIdx.x < p.tiles_m ? (p.tiles_m - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-    const int total_kb = my_tiles * nkb;
-
-    if (warp < kWsProducerWarps) {
-        const uint32_t ring_addr = smem_u32(raw_ring);
-        constexpr int kChunksPerThread = (BM * BK / 4) / (kWsProducerWarps * 32);      // 8
-        auto issue_load = [&](int G) {
-            if (G < total_kb) {
-                const int stage = G % R;
-                mbar_wait(&empty[stage], (uint32_t)(((G / R) & 1) ^ 1));               // MMAs of k-block G-R retired
-                const int tile = blockIdx.x + (G / nkb) * gridDim.x, kb = G % nkb;
-                const int64_t m0 = (int64_t)tile * BM;
-                const uint32_t dst0 = ring_addr + stage * L.raw_bytes;
-#pragma unroll
-                for (int i = 0; i < kChunksPerThread; ++i) {
-                    const int c = t + kWsProducerWarps * 32 * i;
-                    const int r8 = c & 7, kc = (c >> 3) & 7, rg = c >> 6;
-                    const int64_t row = m0 + rg * 8 + r8;
-                    const int k = kb * BK + kc * 4;
-                    uint32_t bytes = 0;
-                    const float *src = p.A;
-                    if (row < p.M && k < p.K) {
-                        bytes = (uint32_t)min(4, p.K - k) * 4u;
-                        src = p.A + row * p.lda + k;
-                    }
-                    cp_async16_zfill(dst0 + c * 16, src, bytes);
-                }
-            }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        };
-#pragma unroll
-        for (int G = 0; G < R - 1; ++G) issue_load(G);
-        for (int G = 0; G < total_kb; ++G) {
-            issue_load(G + R - 1);
-            asm volatile("cp.async.wait_group %0;" ::"n"(R - 1) : "memory");
-            if (G >= 2) mbar_wait(&empty[(G - 2) % R], (uint32_t)(((G - 2) / R) & 1));  // lo[G % 2] no longer read
-            const uint8_t *sraw = raw_ring + (G % R) * L.raw_bytes;
-            uint8_t *slo = lo_bufs + (G & 1) * L.raw_bytes;
-#pragma unroll
-            for (int i = 0; i < kChunksPerThread; ++i) {
-                const int c = t + kWsProducerWarps * 32 * i;
-                const float4 v = *reinterpret_cast<const float4 *>(sraw + c * 16);
-                float4 l;
-                l.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
-                l.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
-                l.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
-                l.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
-                *reinterpret_cast<float4 *>(slo + c * 16) = l;
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&full[G % R]);
-        }
-    } else if (warp == kWsProducerWarps + kWsEpilogueWarps) {
-        if (lane == 0) {
-            const uint32_t idesc = make_idesc(p.un);
-            const uint32_t sbo_b = (L.kpad_b / 4) * 128u;
-            for (int G = 0; G < total_kb; ++G) {
-                const int stage = G % R, it = G / nkb, kb = G % nkb, buf = it & 1;
-                if (kb == 0) mbar_wait(&acc_empty[buf], (uint32_t)(((it >> 1) & 1) ^ 1));
-                mbar_wait(&full[stage], (uint32_t)((G / R) & 1));
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(buf * kMaxUN);
-                const uint32_t a_raw = smem_u32(raw_ring + stage * L.raw_bytes);
-                const uint32_t a_lo = smem_u32(lo_bufs + (G & 1) * L.raw_bytes);
-                const uint32_t b_hi = smem_u32(b_hi_ptr) + (uint32_t)kb * (BK / 4) * 128u, b_lo = b_hi + L.b_bytes;
-                const int steps = kb == nkb - 1 ? last_steps : BK / UMMA_K;
-                for (int j = 0; j < steps; ++j) {
-                    const uint32_t off = (uint32_t)j * 2u * 128u;
-                    const uint64_t dah = make_desc_sbo(a_raw + off, 1024u), dal = make_desc_sbo(a_lo + off, 1024u);
-                    const uint64_t dbh = make_desc_sbo(b_hi + off, sbo_b), dbl = make_desc_sbo(b_lo + off, sbo_b);
-                    umma_tf32(d_tmem, dal, dbh, idesc, (kb | j) != 0);
-                    umma_tf32(d_tmem, dah, dbl, idesc, 1u);
-                    umma_tf32(d_tmem, dah, dbh, idesc, 1u);
-                }
-                umma_commit(&empty[stage]);
-                if (kb == nkb - 1) umma_commit(&acc_full[buf]);
-            }
-        }
-    } else {
-        const int ew = warp - kWsProducerWarps;
-        const int q = warp & 3, half = ew >> 2;
-        const int col_begin = half * (p.un / 2), col_end = (half + 1) * (p.un / 2);
-        const bool vec_ok = (p.ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
-        for (int it = 0; it < my_tiles; ++it) {
-            const int buf = it & 1;
-            const int tile = blockIdx.x + it * gridDim.x;
-            mbar_wait(&acc_full[buf], (uint32_t)((it >> 1) & 1));
-            tc_fence_after();
-            const int64_t row = (int64_t)tile * BM + q * 32 + lane;
-            for (int c0 = col_begin; c0 < col_end; c0 += 8) {
-                uint32_t r[8];
-                const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * kMaxUN + c0);
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                             : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                             : "r"(taddr));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (row < p.M) {
-                    float v[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        v[j] = __uint_as_float(r[j]);
-                        if (p.bias && c0 + j < p.N) v[j] += __ldg(p.bias + c0 + j);
-                        v[j] = apply_act(v[j], p.act);
-                    }
-                    float *dst = p.C + row * p.ldc + c0;
-                    if (vec_ok && c0 + 8 <= p.N) {
-                        *reinterpret_cast<float4 *>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-                        *reinterpret_cast<float4 *>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 8; ++j)
-                            if (c0 + j < p.N) dst[j] = v[j];
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&acc_empty[buf]);
-        }
-    }
-    __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-    }
-}
-
 }  // namespace tc
 }  // namespace tfgk
 
@@ -594,12 +229,9 @@ using namespace tfgk;
 
 extern "C" int tfgk_gemm_tc_f32(const float *A, int64_t lda, const float *B, int64_t ldb, const float *bias, int act,
                                 int32_t M, int32_t N, int32_t K, float *C, int64_t ldc, void *stream) {
-    // Default path for the forward projections; TFGK_GEMM_TC=0 forces the exact-fp32 SIMT kernel.
     // K <= 512: tensor-core accumulation truncates (round-toward-zero), so the error grows ~K^1.5; up to K = 512 it stays
     // below 5e-6 relative (tests/test_gpu_gemm_tc.py), beyond that the SIMT path is used.
-    const char *env = getenv("TFGK_GEMM_TC");
-    const bool enabled = !(env != nullptr && env[0] == '0');
-    if (!enabled || N > tc::kMaxUN || M < 1 || K < 1 || K > 512 || (int64_t)M * K < (1 << 14)) return TFGK_ERR_UNSUPPORTED;
+    if (N > tc::kMaxUN || M < 1 || K < 1 || K > 512 || (int64_t)M * K < (1 << 14)) return TFGK_ERR_UNSUPPORTED;
     tc::Params p;
     p.A = A; p.lda = lda; p.B = B; p.ldb = ldb; p.bias = bias; p.act = act;
     p.M = M; p.N = N; p.K = K; p.C = C; p.ldc = ldc;
@@ -612,36 +244,12 @@ extern "C" int tfgk_gemm_tc_f32(const float *A, int64_t lda, const float *B, int
     TFGK_CUDA(cudaGetDevice(&dev));
     TFGK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int grid = p.tiles_m < sms ? p.tiles_m : sms;       // persistent: one CTA per SM
-    const char *impl = getenv("TFGK_GEMM_TC_IMPL");
-    if (impl && impl[0] == 'd') {             // "deep": warp-specialised with the deep raw ring
-        const tc::SmemPlanDeep LD(p.un, K);
-        if (LD.ring >= 3 && (2u * LD.b_bytes) % 1024u == 0) {
-#define TFGK_LAUNCH_DEEP(RR)                                                                                              \
-            TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_deep_kernel<RR>, LD.total)); \
-            tc::gemm_tf32x3_deep_kernel<RR><<<grid, tc::kWsThreads, LD.total, as_stream(stream)>>>(p)
-            if (LD.ring == 5) { TFGK_LAUNCH_DEEP(5); } else if (LD.ring == 4) { TFGK_LAUNCH_DEEP(4); } else { TFGK_LAUNCH_DEEP(3); }
-#undef TFGK_LAUNCH_DEEP
-            TFGK_LAUNCH_CHECK();
-            return TFGK_OK;
-        }
-    }
-    if (!(impl && impl[0] == 's')) {          // default: warp-specialised; "sync" selects the __syncthreads variant
-        if (L.stages == 3) {
-            TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_ws_kernel<3>, L.total));
-            tc::gemm_tf32x3_ws_kernel<3><<<grid, tc::kWsThreads, L.total, as_stream(stream)>>>(p);
-        } else {
-            TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_ws_kernel<2>, L.total));
-            tc::gemm_tf32x3_ws_kernel<2><<<grid, tc::kWsThreads, L.total, as_stream(stream)>>>(p);
-        }
-        TFGK_LAUNCH_CHECK();
-        return TFGK_OK;
-    }
     if (L.stages == 3) {
-        TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_kernel<3>, L.total));
-        tc::gemm_tf32x3_kernel<3><<<grid, tc::kThreads, L.total, as_stream(stream)>>>(p);
+        TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_ws_kernel<3>, L.total));
+        tc::gemm_tf32x3_ws_kernel<3><<<grid, tc::kWsThreads, L.total, as_stream(stream)>>>(p);
     } else {
-        TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_kernel<2>, L.total));
-        tc::gemm_tf32x3_kernel<2><<<grid, tc::kThreads, L.total, as_stream(stream)>>>(p);
+        TFGK_CUDA(ensure_dynamic_smem(tc::gemm_tf32x3_ws_kernel<2>, L.total));
+        tc::gemm_tf32x3_ws_kernel<2><<<grid, tc::kWsThreads, L.total, as_stream(stream)>>>(p);
     }
     TFGK_LAUNCH_CHECK();
     return TFGK_OK;

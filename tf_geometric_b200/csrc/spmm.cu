@@ -11,7 +11,6 @@
 //
 // Algorithmic bytes per launch (DESIGN.md): E*(4*D + 4 [+4 weighted]) + N*(4*D + 8).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace tfgk {
 
@@ -175,309 +174,14 @@ __global__ void __launch_bounds__(kSpmmThreads) spmm_kernel(const SpmmParams p) 
     }
 }
 
-
 // ------------------------------------------------------------------------------------------------------------
-// TMA variant (D % 4 == 0): the neighbour rows are pulled by the bulk-copy engine (cp.async.bulk, SASS UBLKCP)
-// straight into a per-warp shared-memory ring, 32 rows per stage, completion tracked by an mbarrier transaction
-// count.  A warp owns a block of consecutive destination rows, i.e. a CONTIGUOUS range of CSR edges, and streams
-// that range in 32-edge chunks regardless of row boundaries: chunk j+1 is in flight while chunk j is reduced, so
-// the memory pipe never drains at a row change and no registers are spent on in-flight data.
-// Accumulation order and rounding are identical to spmm_kernel (CSR order, separate mul/add) => same bits.
-// ------------------------------------------------------------------------------------------------------------
-constexpr int kBulkChunk = 32;        // edges (= bulk copies) per stage, one per lane
-constexpr int kBulkRowsPerWarp = 32;  // destination rows per warp
-
-__device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    for (uint32_t spin = 0; !done; ++spin) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (spin > (1u << 28)) __trap();     // a lost transaction becomes a launch failure, never a hang
-    }
-}
-
-template <int NC, bool IS_MAX>
-__global__ void __launch_bounds__(256) spmm_bulk_kernel(const SpmmParams p, int warps_per_cta, uint32_t row_bytes) {
-    extern __shared__ __align__(128) uint8_t smem_raw[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    // layout: [warps][2 stages][32 rows][row_bytes] then [warps][2] mbarriers
-    const uint32_t stage_bytes = kBulkChunk * row_bytes;
-    uint8_t *my_buf = smem_raw + (size_t)warp * 2 * stage_bytes;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw + (size_t)warps_per_cta * 2 * stage_bytes) + warp * 2;
-    const uint32_t bar0 = smem_addr(bars);
-    if (lane == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0 + 8));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-
-    const int64_t r0 = ((int64_t)blockIdx.x * warps_per_cta + warp) * kBulkRowsPerWarp;
-    if (r0 >= p.n_dst) return;
-    const int64_t r1 = min((int64_t)p.n_dst, r0 + kBulkRowsPerWarp);
-    // lane l keeps rowptr[r0+l] and rowptr[r0+l+1] (clamped): ends of the warp's rows, broadcast by shuffle
-    const int64_t rp_lo = p.rowptr[min(r0 + lane, r1)];
-    const int64_t rp_hi = p.rowptr[min(r0 + lane + 1, r1)];
-    const int64_t e_begin = __shfl_sync(0xffffffffu, rp_lo, 0);
-    const int64_t e_end = p.rowptr[r1];
-    const int n_edges = (int)(e_end - e_begin);
-    const int n_chunks = (n_edges + kBulkChunk - 1) / kBulkChunk;
-    const bool weighted = p.w != nullptr;
-    const uint32_t buf_addr = smem_addr(my_buf);
-
-    float wreg[2] = {1.0f, 1.0f};
-    auto issue = [&](int j) {
-        const int stage = j & 1;
-        const int e = j * kBulkChunk + lane;
-        const int nb = min(kBulkChunk, n_edges - j * kBulkChunk);
-        const uint32_t bar = bar0 + 8 * stage;
-        if (lane == 0)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)nb * row_bytes) : "memory");
-        float wv = 1.0f;
-        if (e < n_edges) {
-            const int c = ld_stream_i32(p.col + e_begin + e);
-            if (weighted) wv = ld_stream_f32(p.w + e_begin + e);
-            const float *src = p.h + (int64_t)c * p.ldh;
-            const uint32_t dst = buf_addr + stage * stage_bytes + lane * row_bytes;
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(dst), "l"(src), "r"(row_bytes), "r"(bar) : "memory");
-        }
-        wreg[stage] = wv;
-    };
-
-    int coff[NC];
-    bool cok[NC];
-    float acc[NC][4];
-#pragma unroll
-    for (int k = 0; k < NC; ++k) {
-        coff[k] = (lane + 32 * k) * 4;
-        cok[k] = coff[k] < p.D;
-#pragma unroll
-        for (int x = 0; x < 4; ++x) acc[k][x] = IS_MAX ? -FLT_MAX : 0.0f;
-    }
-
-    int64_t r = r0;
-    int64_t row_end = __shfl_sync(0xffffffffu, rp_hi, 0) - e_begin;   // end of row r, relative to e_begin
-    const bool is_mean = p.reduce == TFGK_REDUCE_MEAN;
-
-    auto finalize_row = [&]() {
-        const int64_t row_start = __shfl_sync(0xffffffffu, rp_lo, (int)(r - r0));
-        const int deg = (int)(row_end + e_begin - row_start);
-        const float cnt = (float)max(deg, 1);
-#pragma unroll
-        for (int k = 0; k < NC; ++k) {
-            if (cok[k]) {
-                float ad[4], bs[4], o[4];
-                if (p.addend) load_vec<4>(p.addend + r * p.ld_addend + coff[k], ad);
-                if (p.bias) load_vec<4>(p.bias + coff[k], bs);
-#pragma unroll
-                for (int x = 0; x < 4; ++x) {
-                    float a = acc[k][x];
-                    if (is_mean) a = __fdiv_rn(a, cnt);
-                    if (p.addend) a = __fadd_rn(__fmul_rn(a, p.alpha), __fmul_rn(ad[x], p.beta));
-                    else if (p.alpha != 1.0f) a = __fmul_rn(a, p.alpha);
-                    if (p.bias) a = __fadd_rn(a, bs[x]);
-                    o[x] = apply_act(a, p.act);
-                    acc[k][x] = IS_MAX ? -FLT_MAX : 0.0f;
-                }
-                store_vec<4>(p.out + r * p.ldo + coff[k], o);
-            }
-        }
-        ++r;
-        if (r < r1) row_end = __shfl_sync(0xffffffffu, rp_hi, (int)(r - r0)) - e_begin;
-    };
-
-    if (n_chunks > 0) issue(0);
-    for (int j = 0; j < n_chunks; ++j) {
-        __syncwarp();                                   // every lane is done reading the stage issue(j+1) overwrites
-        if (j + 1 < n_chunks) issue(j + 1);
-        const int stage = j & 1;
-        mbar_wait_parity(bar0 + 8 * stage, (uint32_t)(j >> 1) & 1u);
-        const int nb = min(kBulkChunk, n_edges - j * kBulkChunk);
-        const uint8_t *sbuf = my_buf + stage * stage_bytes;
-        const float wmine = wreg[stage];
-        for (int i = 0; i < nb; ++i) {
-            const int64_t e = (int64_t)j * kBulkChunk + i;
-            while (e == row_end) finalize_row();        // also steps over empty rows
-            const float we = __shfl_sync(0xffffffffu, wmine, i);
-#pragma unroll
-            for (int k = 0; k < NC; ++k) {
-                if (cok[k]) {
-                    const float4 v = *reinterpret_cast<const float4 *>(sbuf + (size_t)i * row_bytes + coff[k] * 4);
-                    const float m0 = __fmul_rn(v.x, we), m1 = __fmul_rn(v.y, we), m2 = __fmul_rn(v.z, we), m3 = __fmul_rn(v.w, we);
-                    acc[k][0] = IS_MAX ? fmaxf(acc[k][0], m0) : __fadd_rn(acc[k][0], m0);
-                    acc[k][1] = IS_MAX ? fmaxf(acc[k][1], m1) : __fadd_rn(acc[k][1], m1);
-                    acc[k][2] = IS_MAX ? fmaxf(acc[k][2], m2) : __fadd_rn(acc[k][2], m2);
-                    acc[k][3] = IS_MAX ? fmaxf(acc[k][3], m3) : __fadd_rn(acc[k][3], m3);
-                }
-            }
-        }
-    }
-    while (r < r1) finalize_row();                      // last row and trailing empty rows
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// Streaming variant (float4 rows): a warp owns kStreamRows consecutive destination rows = one CONTIGUOUS range of CSR
-// edges, and walks that range in rounds of U edges with two register buffers: the gathers of round g+1 are issued
-// before round g is reduced, and the (col, w) of the next 32-edge chunk are fetched one chunk ahead.  The memory
-// pipe therefore never drains at a row boundary or while indices are being fetched - by Little's law the achieved
-// bandwidth is (bytes in flight) / (loaded latency), and this keeps 8-16 rows in flight per warp all the time instead
-// of 8 for a fraction of it.  Rounding and order are unchanged (CSR order, separate mul/add) => same bits.
-// ------------------------------------------------------------------------------------------------------------
-constexpr int kStreamRows = 16;        // destination rows per warp (their finished sums wait in shared memory)
-constexpr int kStreamThreads = 128;
-constexpr int kStreamWarps = kStreamThreads / 32;
-
-template <bool IS_MAX, int U, int MINB>
-__global__ void __launch_bounds__(kStreamThreads, MINB) spmm_stream_kernel(const SpmmParams p) {
-    static_assert(32 % U == 0, "a round must not straddle an index chunk");
-    constexpr int RPC = 32 / U;                 // rounds per 32-edge index chunk
-    __shared__ float4 stash[kStreamWarps][kStreamRows][32];      // finished row sums, one float4 per lane
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t r0 = ((int64_t)blockIdx.x * kStreamWarps + warp) * kStreamRows;
-    if (r0 >= p.n_dst) return;
-    const int n_rows = (int)min((int64_t)kStreamRows, (int64_t)p.n_dst - r0);
-    // lane l < n_rows describes row r0 + l
-    const int64_t rp_lo = p.rowptr[r0 + min(lane, n_rows)];
-    const int64_t rp_hi = p.rowptr[r0 + min(lane + 1, n_rows)];
-    const int64_t e_begin = __shfl_sync(0xffffffffu, rp_lo, 0);
-    const int n_edges = (int)(__shfl_sync(0xffffffffu, rp_hi, n_rows - 1) - e_begin);
-    const int my_end = (int)(rp_hi - e_begin);                   // end of row `lane`, relative
-    const int my_deg = (int)(rp_hi - rp_lo);
-    const uint32_t nonempty = __ballot_sync(0xffffffffu, lane < n_rows && my_deg > 0);
-    const bool weighted = p.w != nullptr;
-    const float *__restrict__ h = p.h;
-    const int coff = lane * 4;
-    const bool cok = coff < p.D;
-    const float init = IS_MAX ? -FLT_MAX : 0.0f;
-
-#pragma unroll
-    for (int i = 0; i < kStreamRows; ++i) stash[warp][i][lane] = make_float4(init, init, init, init);
-
-    float a0 = init, a1 = init, a2 = init, a3 = init;
-    int rel = nonempty ? __ffs(nonempty) - 1 : n_rows;           // current (non-empty) row
-    int row_end = rel < n_rows ? __shfl_sync(0xffffffffu, my_end, rel & 31) : -1;
-
-    auto load_chunk = [&](int c, int &ci, float &wi) {
-        const int e = c * 32 + lane;
-        ci = 0;
-        wi = 1.0f;
-        if (e < n_edges) {
-            ci = ld_stream_i32(p.col + e_begin + e);
-            if (weighted) wi = ld_stream_f32(p.w + e_begin + e);
-        }
-    };
-    auto issue = [&](int g, int ci, float4 (&buf)[U]) {
-        const int base = (g % RPC) * U;
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const int c = __shfl_sync(0xffffffffu, ci, base + u);
-            if (g * U + u < n_edges && cok) buf[u] = __ldg(reinterpret_cast<const float4 *>(h + (int64_t)c * p.ldh + coff));
-        }
-    };
-    auto consume = [&](int g, float wi, const float4 (&buf)[U]) {
-        const int base = (g % RPC) * U;
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const int e = g * U + u;
-            const float we = __shfl_sync(0xffffffffu, wi, base + u);
-            if (e < n_edges) {
-                const float m0 = __fmul_rn(buf[u].x, we), m1 = __fmul_rn(buf[u].y, we);
-                const float m2 = __fmul_rn(buf[u].z, we), m3 = __fmul_rn(buf[u].w, we);
-                a0 = IS_MAX ? fmaxf(a0, m0) : __fadd_rn(a0, m0);
-                a1 = IS_MAX ? fmaxf(a1, m1) : __fadd_rn(a1, m1);
-                a2 = IS_MAX ? fmaxf(a2, m2) : __fadd_rn(a2, m2);
-                a3 = IS_MAX ? fmaxf(a3, m3) : __fadd_rn(a3, m3);
-                if (e + 1 == row_end) {          // last edge of the row: park the sum, move to the next non-empty row
-                    stash[warp][rel][lane] = make_float4(a0, a1, a2, a3);
-                    a0 = a1 = a2 = a3 = init;
-                    const uint32_t rest = rel < 31 ? (nonempty >> (rel + 1)) : 0u;
-                    rel = rest ? rel + __ffs(rest) : n_rows;
-                    row_end = rel < n_rows ? __shfl_sync(0xffffffffu, my_end, rel & 31) : -1;
-                }
-            }
-        }
-    };
-
-    float4 buf0[U], buf1[U];
-    int ca, cb;
-    float wa, wb;
-    load_chunk(0, ca, wa);
-    load_chunk(1, cb, wb);
-    issue(0, ca, buf0);
-    const int n_rounds = (n_edges + U - 1) / U;
-    // two rounds per iteration (buf0 <-> buf1); the chunk registers are picked with selects, not by unrolling
-    for (int g = 0; g < n_rounds; g += 2) {
-        {
-            const int cn = (g + 1) / RPC, cc = g / RPC;
-            issue(g + 1, (cn & 1) ? cb : ca, buf1);
-            consume(g, (cc & 1) ? wb : wa, buf0);
-            if ((g + 1) % RPC == 0) { if (cc & 1) load_chunk(cc + 2, cb, wb); else load_chunk(cc + 2, ca, wa); }
-        }
-        {
-            const int cn = (g + 2) / RPC, cc = (g + 1) / RPC;
-            issue(g + 2, (cn & 1) ? cb : ca, buf0);
-            consume(g + 1, (cc & 1) ? wb : wa, buf1);
-            if ((g + 2) % RPC == 0) { if (cc & 1) load_chunk(cc + 2, cb, wb); else load_chunk(cc + 2, ca, wa); }
-        }
-    }
-
-    // epilogue for the warp's rows: uniform loop, coalesced 512-byte stores
-    const bool is_mean = p.reduce == TFGK_REDUCE_MEAN;
-    float bs[4] = {0.f, 0.f, 0.f, 0.f};
-    if (p.bias && cok) load_vec<4>(p.bias + coff, bs);
-    for (int i = 0; i < n_rows; ++i) {
-        const float cnt = (float)max(__shfl_sync(0xffffffffu, my_deg, i), 1);     // every lane takes part in the shuffle
-        if (!cok) continue;
-        const float4 v = stash[warp][i][lane];
-        float a[4] = {v.x, v.y, v.z, v.w}, ad[4], o[4];
-        const int64_t r = r0 + i;
-        if (p.addend) load_vec<4>(p.addend + r * p.ld_addend + coff, ad);
-#pragma unroll
-        for (int x = 0; x < 4; ++x) {
-            float t = a[x];
-            if (is_mean) t = __fdiv_rn(t, cnt);
-            if (p.addend) t = __fadd_rn(__fmul_rn(t, p.alpha), __fmul_rn(ad[x], p.beta));
-            else if (p.alpha != 1.0f) t = __fmul_rn(t, p.alpha);
-            if (p.bias) t = __fadd_rn(t, bs[x]);
-            o[x] = apply_act(t, p.act);
-        }
-        store_vec<4>(p.out + r * p.ldo + coff, o);
-    }
-}
-
-template <int U, int MINB>
-static int launch_spmm_stream(const SpmmParams &p, cudaStream_t st) {
-    const int64_t rows_per_cta = (int64_t)kStreamWarps * kStreamRows;
-    const unsigned blocks = (unsigned)ceil_div64(p.n_dst, rows_per_cta);
-    if (p.reduce == TFGK_REDUCE_MAX) spmm_stream_kernel<true, U, MINB><<<blocks, kStreamThreads, 0, st>>>(p);
-    else spmm_stream_kernel<false, U, MINB><<<blocks, kStreamThreads, 0, st>>>(p);
-    TFGK_LAUNCH_CHECK();
-    return TFGK_OK;
-}
-
-static int dispatch_spmm_stream(const SpmmParams &p, cudaStream_t st) {
-    if (p.D > 128) return TFGK_ERR_UNSUPPORTED;            // wider rows: the per-row kernel (register budget)
-    const char *cfg = getenv("TFGK_SPMM_STREAM_CFG");     // tuning knob: "8x4" (default), "8x5", "4x8", "16x2"
-    if (cfg && cfg[0] == '4') return launch_spmm_stream<4, 8>(p, st);
-    if (cfg && cfg[0] == '1') return launch_spmm_stream<16, 2>(p, st);
-    if (cfg && cfg[0] == '8' && cfg[2] == '5') return launch_spmm_stream<8, 5>(p, st);
-    return launch_spmm_stream<8, 4>(p, st);
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// cp.async variant.  Register double-buffering cannot overlap two gather rounds: a warp has six counting scoreboard
+// cp.async ring.  Register double-buffering cannot overlap two gather rounds: a warp has six counting scoreboard
 // slots, ptxas puts the loads of both rounds on the same slots, and the first use of round g then also waits for
 // round g+1 (decoded from SASS, profiles/r1_notes.md).  LDGSTS copies are tracked by commit groups instead, so a
 // per-warp shared-memory ring of S stages x U rows keeps (S-1)*U rows in flight per warp with no register cost.
 // Each lane copies - and later reads back - only its own 16-byte slices: shared memory is used as an asynchronous
-// extension of the register file, no cross-lane traffic, no barriers.  Edge streaming as above: a warp owns
-// kAsyncRows consecutive rows = a contiguous CSR range.  Same rounding and order => same bits.
+// extension of the register file, no cross-lane traffic, no barriers.  Edge streaming: a warp owns kAsyncRows consecutive
+// rows = a contiguous CSR range, walked in rounds of U edges across row boundaries.  Same rounding and order => same bits.
 // ------------------------------------------------------------------------------------------------------------
 constexpr int kAsyncRows = 32;
 constexpr int kAsyncWarps = 4;
@@ -657,13 +361,22 @@ __global__ void __launch_bounds__(kAsyncWarps * 32) spmm_async_kernel(const Spmm
 // arithmetic as spmm_async_kernel, but a round of U = 4 edges is ONE instruction
 //     cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4 [ring stage], [tensor map of h, {0, c0, c1, c2, c3}], [mbarrier]
 // issued by one lane: the TMA unit fetches the four neighbour rows (box = D columns x 1 row each) and completes the
-// stage's mbarrier with 4 * row_bytes transaction bytes.  That is a quarter of the TMA issue rate that sank the 1-D
-// cp.async.bulk variant (one 512-byte copy per row, spmm_bulk_kernel) and frees the 4 LDGSTS issue slots per lane and
-// round of the cp.async ring.  Each warp owns S mbarriers; a stage is re-armed only after every lane has read it
-// (__syncwarp before the elected lane issues).  Rows beyond the edge range repeat a valid row id (the bytes still count
+// stage's mbarrier with 4 * row_bytes transaction bytes.  That is a quarter of the TMA issues of a 1-D cp.async.bulk
+// copy per row, and frees the 4 LDGSTS issue slots per lane and round of the cp.async ring.  Each warp owns S mbarriers;
+// a stage is re-armed only after every lane has read it (__syncwarp before the elected lane issues).  Rows beyond the edge range repeat a valid row id (the bytes still count
 // towards the stage's transaction total) and are ignored by the consumer.  Same rounding and order => same bits.
 // ------------------------------------------------------------------------------------------------------------
-struct alignas(64) TensorMap { uint64_t opaque[16]; };      // CUtensorMap (128 bytes), filled by the driver on the host
+__device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) {
+    uint32_t done = 0;
+    for (uint32_t spin = 0; !done; ++spin) {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+        if (spin > (1u << 28)) __trap();     // a lost transaction becomes a launch failure, never a hang
+    }
+}
 
 __device__ __forceinline__ void tma_gather4(uint32_t dst, const TensorMap *map, int c0, int c1, int c2, int c3, uint32_t bar) {
     asm volatile(
@@ -893,31 +606,6 @@ static int launch_spmm_async(const SpmmParams &p, cudaStream_t st) {
     return TFGK_OK;
 }
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda)
-typedef int (*EncodeTiledFn)(void *map, int dtype, uint32_t rank, void *base, const uint64_t *dims, const uint64_t *strides,
-                             const uint32_t *box, const uint32_t *elem_strides, int interleave, int swizzle, int l2promo,
-                             int oob_fill);
-
-static int make_row_tensor_map(TensorMap *out, const float *h, int64_t ldh, int64_t n_rows, int32_t D) {
-    static EncodeTiledFn encode = nullptr;
-    if (encode == nullptr) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        TFGK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (fn == nullptr || qres != cudaDriverEntryPointSuccess)
-            return set_error(TFGK_ERR_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
-        encode = reinterpret_cast<EncodeTiledFn>(fn);
-    }
-    const uint64_t dims[2] = {(uint64_t)D, (uint64_t)n_rows};
-    const uint64_t strides[1] = {(uint64_t)ldh * sizeof(float)};          // byte stride of dimension 1 (rows)
-    const uint32_t box[2] = {(uint32_t)D, 1u};                            // gather4: 1 in the gathered dimension
-    const uint32_t elem[2] = {1u, 1u};
-    // CU_TENSOR_MAP_DATA_TYPE_FLOAT32 = 7, INTERLEAVE_NONE = 0, SWIZZLE_NONE = 0, L2_PROMOTION_L2_128B = 2, OOB_FILL_NONE = 0
-    const int rc = encode(out, 7, 2, const_cast<float *>(h), dims, strides, box, elem, 0, 0, 2, 0);
-    if (rc != 0) return set_error(TFGK_ERR_UNSUPPORTED, "cuTensorMapEncodeTiled failed with CUresult %d", rc);
-    return TFGK_OK;
-}
-
 template <int S>
 static int launch_spmm_gather4(const SpmmParams &p, int64_t h_rows, cudaStream_t st) {
     if (p.D > 256 || p.D % 4 != 0 || p.ldh % 4 != 0) return TFGK_ERR_UNSUPPORTED;
@@ -947,69 +635,11 @@ static int launch_spmm_gather4(const SpmmParams &p, int64_t h_rows, cudaStream_t
     return TFGK_OK;
 }
 
+// float4 rows of 257..512 columns (gather4 takes up to 256)
 static int dispatch_spmm_async(const SpmmParams &p, cudaStream_t st) {
     const int lanes = (p.D + 3) / 4;
-    const char *cfg = getenv("TFGK_SPMM_ASYNC_CFG");      // tuning knob for NC == 1, "UxS"; default 4x3
-    if (lanes <= 32) {
-        if (cfg && cfg[0] == '8' && cfg[2] == '4') return launch_spmm_async<1, 8, 4>(p, st);
-        if (cfg && cfg[0] == '8' && cfg[2] == '2') return launch_spmm_async<1, 8, 2>(p, st);
-        if (cfg && cfg[0] == '8' && cfg[2] == '6') return launch_spmm_async<1, 8, 6>(p, st);
-        if (cfg && cfg[0] == '8' && cfg[2] == '3') return launch_spmm_async<1, 8, 3>(p, st);
-        if (cfg && cfg[0] == '4' && cfg[2] == '4') return launch_spmm_async<1, 4, 4>(p, st);
-        if (cfg && cfg[0] == '4' && cfg[2] == '6') return launch_spmm_async<1, 4, 6>(p, st);
-        if (cfg && cfg[0] == '2' && cfg[2] == '6') return launch_spmm_async<1, 2, 6>(p, st);
-        if (cfg && cfg[0] == '2' && cfg[2] == '4') return launch_spmm_async<1, 2, 4>(p, st);
-        return launch_spmm_async<1, 4, 3>(p, st);      // 99% of the measured HBM peak at D=128 (profiles/r1_kernel_variants_spmm_async.json)
-    }
-    if (lanes <= 64) return launch_spmm_async<2, 4, 4>(p, st);
     if (lanes <= 96) return launch_spmm_async<3, 4, 3>(p, st);
     return launch_spmm_async<4, 2, 4>(p, st);
-}
-
-// Default kernel: the TMA tile::gather4 ring with three stages for every float4-aligned width up to 256 columns
-// (profiles/r2_kernel_variants_final.json: D = 128 9.55 ms against 9.87 ms for the cp.async ring, D = 100 9.51 against 10.24;
-// three stages beat four, six and eight, which cost resident warps).  TFGK_SPMM_IMPL=async keeps the cp.async ring, which is also
-// the fallback when the driver entry point for tensor maps is unavailable.
-static bool spmm_prefers_gather4(int D) { return D >= 32 && D <= 256; }
-
-static int spmm_impl_choice() {
-    // 0 = register-staged LDG gather, 1 = TMA bulk gather.  TFGK_SPMM_IMPL overrides (read per call: cheap).
-    const char *e = getenv("TFGK_SPMM_IMPL");
-    if (e && e[0] == 'b') return 1;
-    if (e && e[0] == 's') return 2;
-    if (e && (e[0] == 'g' || e[0] == 't')) return 4;      // "gather4" / "tma": TMA tile::gather4 ring
-    if (e && e[0] == 'l') return 0;
-    if (e && e[0] == 'a') return 3;      // "async": the cp.async ring for every shape
-    return 5;                            // default: by row shape (spmm_prefers_gather4); "ldg" / "stream" / "bulk" are the measured alternatives
-}
-
-template <int NC>
-static int launch_spmm_bulk(const SpmmParams &p, cudaStream_t st) {
-    const uint32_t row_bytes = (uint32_t)p.D * 4u;
-    const size_t per_warp = 2u * kBulkChunk * row_bytes + 16;
-    int warps = (int)((220 * 1024) / per_warp);
-    if (warps > 8) warps = 8;
-    if (warps < 1) return TFGK_ERR_UNSUPPORTED;
-    const size_t smem = (size_t)warps * per_warp;
-    const int64_t rows_per_cta = (int64_t)warps * kBulkRowsPerWarp;
-    const unsigned blocks = (unsigned)ceil_div64(p.n_dst, rows_per_cta);
-    if (p.reduce == TFGK_REDUCE_MAX) {
-        TFGK_CUDA(ensure_dynamic_smem(spmm_bulk_kernel<NC, true>, smem));
-        spmm_bulk_kernel<NC, true><<<blocks, warps * 32, smem, st>>>(p, warps, row_bytes);
-    } else {
-        TFGK_CUDA(ensure_dynamic_smem(spmm_bulk_kernel<NC, false>, smem));
-        spmm_bulk_kernel<NC, false><<<blocks, warps * 32, smem, st>>>(p, warps, row_bytes);
-    }
-    TFGK_LAUNCH_CHECK();
-    return TFGK_OK;
-}
-
-static int dispatch_spmm_bulk(const SpmmParams &p, cudaStream_t st) {
-    const int lanes = (p.D + 3) / 4;
-    if (lanes <= 32) return launch_spmm_bulk<1>(p, st);
-    if (lanes <= 64) return launch_spmm_bulk<2>(p, st);
-    if (lanes <= 96) return launch_spmm_bulk<3>(p, st);
-    return launch_spmm_bulk<4>(p, st);
 }
 
 template <int VEC, int G, int NC, int U>
@@ -1074,8 +704,7 @@ extern "C" int tfgk_spmm_f32(const int64_t *rowptr, const int32_t *col, const fl
         p.task_slot = nullptr; p.n_hubs = 0; p.hub_row = nullptr; p.hub_slot0 = nullptr; p.hub_nslots = nullptr;
         p.scratch = nullptr;
         // the plan applies when the whole width runs in one launch of the streaming kernel (scratch rows are D wide)
-        const bool use_plan = plan != nullptr && plan->n_tasks > 0 && vec4 && D >= 32 && D <= cols_per_launch &&
-                              (spmm_impl_choice() >= 3);
+        const bool use_plan = plan != nullptr && plan->n_tasks > 0 && vec4 && D >= 32 && D <= cols_per_launch;
         if (use_plan) {
             p.n_tasks = plan->n_tasks; p.task_row = plan->task_row; p.task_nrows = plan->task_nrows;
             p.task_e0 = plan->task_e0; p.task_e1 = plan->task_e1; p.task_slot = plan->task_slot;
@@ -1083,30 +712,18 @@ extern "C" int tfgk_spmm_f32(const int64_t *rowptr, const int32_t *col, const fl
             p.hub_nslots = plan->hub_nslots; p.scratch = plan->scratch;
         }
         const int lanes = (p.D + vec - 1) / vec;
-        const int choice = spmm_impl_choice() == 5 ? (spmm_prefers_gather4(p.D) ? 4 : 3) : spmm_impl_choice();
-        if (vec4 && p.D >= 32 && choice == 4) {
+        // Float4 rows of 32..256 columns: the TMA tile::gather4 ring with three stages (profiles/r2_kernel_variants_final.json,
+        // B200: D = 128 9.55 ms against 9.87 ms for the cp.async ring, D = 100 9.51 against 10.24; three stages beat four, six
+        // and eight, which cost resident warps).  Wider float4 rows: the cp.async ring.  Everything else, and any row when no
+        // tensor map can be encoded: the per-row LDG kernel.
+        if (vec4 && p.D >= 32 && p.D <= 256) {
             // the ABI does not carry the number of source rows: the tensor map is bounded by the index type instead
             // (column ids were validated against n_cols when the CSR was built)
-            const char *cfg = getenv("TFGK_SPMM_GATHER4_STAGES");
-            const int st = cfg ? atoi(cfg) : 3;
-            const int rcg = st == 2 ? launch_spmm_gather4<2>(p, (int64_t)1 << 31, as_stream(stream))
-                          : st == 3 ? launch_spmm_gather4<3>(p, (int64_t)1 << 31, as_stream(stream))
-                          : st == 6 ? launch_spmm_gather4<6>(p, (int64_t)1 << 31, as_stream(stream))
-                          : st == 8 ? launch_spmm_gather4<8>(p, (int64_t)1 << 31, as_stream(stream))
-                                    : launch_spmm_gather4<4>(p, (int64_t)1 << 31, as_stream(stream));
+            const int rcg = launch_spmm_gather4<3>(p, (int64_t)1 << 31, as_stream(stream));
             if (rcg != TFGK_ERR_UNSUPPORTED) { if (rcg != TFGK_OK) return rcg; continue; }
-        }
-        if (vec4 && p.D >= 32 && (choice == 3 || choice == 4)) {
+        } else if (vec4 && p.D > 256) {
             const int rca = dispatch_spmm_async(p, as_stream(stream));
             if (rca != TFGK_ERR_UNSUPPORTED) { if (rca != TFGK_OK) return rca; continue; }
-        }
-        if (vec4 && p.D >= 32 && choice == 2) {
-            const int rcs = dispatch_spmm_stream(p, as_stream(stream));
-            if (rcs != TFGK_ERR_UNSUPPORTED) { if (rcs != TFGK_OK) return rcs; continue; }
-        }
-        if (vec4 && p.D >= 32 && choice == 1) {
-            const int rcb = dispatch_spmm_bulk(p, as_stream(stream));
-            if (rcb != TFGK_ERR_UNSUPPORTED) { if (rcb != TFGK_OK) return rcb; continue; }
         }
         const int rc = vec4 ? dispatch_spmm<4>(p, lanes, as_stream(stream)) : dispatch_spmm<1>(p, lanes, as_stream(stream));
         if (rc != TFGK_OK) return rc;

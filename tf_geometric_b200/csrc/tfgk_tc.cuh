@@ -8,7 +8,6 @@ namespace tc {
 constexpr int BM = 128;            // UMMA_M
 constexpr int BK = 32;             // K elements per smem stage (8 core matrices of 16 B along K)
 constexpr int UMMA_K = 8;          // tf32
-constexpr int kThreads = 256;
 constexpr int kMaxUN = 256;
 constexpr int kTmemCols = 512;
 constexpr uint32_t kSpinLimit = 1u << 28;

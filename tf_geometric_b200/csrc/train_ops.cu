@@ -4,7 +4,6 @@
 // pass (and its transpose for the scatter-shaped gradients), deterministic, no atomics.
 #include "common.cuh"
 #include "rng.cuh"
-#include <stdlib.h>
 
 namespace tfgk {
 namespace {
@@ -288,15 +287,8 @@ int tfgk_spmm_heads_f32(const int64_t *rowptr, const int32_t *col, const int32_t
     const bool fast = mode == TFGK_HEADS_SPLIT && (int64_t)H * dh == 128 && dh % 4 == 0 && aligned16(src) && aligned16(out) &&
                       lds % 4 == 0 && ldo % 4 == 0 && (!bias || aligned16(bias));
     if (fast) {
-        const char *cfg = getenv("TFGK_SPMM_HEADS_CFG");       // rows in flight per warp: "8" or the default 4
-        const bool wide = cfg && cfg[0] == '8';
-        if (drop_rate > 0.0f) {
-            if (wide) spmm_heads128_kernel<8, true><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
-            else spmm_heads128_kernel<4, true><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
-        } else {
-            if (wide) spmm_heads128_kernel<8, false><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
-            else spmm_heads128_kernel<4, false><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
-        }
+        if (drop_rate > 0.0f) spmm_heads128_kernel<4, true><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
+        else spmm_heads128_kernel<4, false><<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
     } else
         spmm_heads_kernel<<<blocks, kTrainThreads, 0, as_stream(stream)>>>(p);
     TFGK_LAUNCH_CHECK();
@@ -323,20 +315,8 @@ int tfgk_gat_softmax_bwd_f32(const int64_t *rowptr, const int32_t *col, const fl
     const bool fast = p.split && (int64_t)H * dv == 128 && dv % 4 == 0 && pow2(dv >> 2) && aligned16(G) && aligned16(V) &&
                       ldg % 4 == 0 && ldv % 4 == 0;
     if (fast) {
-        const char *cfg = getenv("TFGK_GAT_BWD_CFG");          // "UxB": rows in flight x resident CTAs per SM; default 4x4
-        const int sel = (cfg && cfg[0] == '8' && cfg[2] == '3') ? 1 : (cfg && cfg[0] == '4' && cfg[2] == '5') ? 2
-                        : (cfg && cfg[0] == '8' && cfg[2] == '4') ? 3 : 0;
-        cudaStream_t st = as_stream(stream);
-#define TFGK_LAUNCH_BWD(UU, BB)                                                                         \
-    do {                                                                                                \
-        if (drop_rate > 0.0f) gat_softmax_bwd128_kernel<UU, BB, true><<<blocks, kTrainThreads, smem, st>>>(p);  \
-        else gat_softmax_bwd128_kernel<UU, BB, false><<<blocks, kTrainThreads, smem, st>>>(p);          \
-    } while (0)
-        if (sel == 1) TFGK_LAUNCH_BWD(8, 3);
-        else if (sel == 2) TFGK_LAUNCH_BWD(4, 5);
-        else if (sel == 3) TFGK_LAUNCH_BWD(8, 4);
-        else TFGK_LAUNCH_BWD(4, 4);
-#undef TFGK_LAUNCH_BWD
+        if (drop_rate > 0.0f) gat_softmax_bwd128_kernel<4, 4, true><<<blocks, kTrainThreads, smem, as_stream(stream)>>>(p);
+        else gat_softmax_bwd128_kernel<4, 4, false><<<blocks, kTrainThreads, smem, as_stream(stream)>>>(p);
     } else
         gat_softmax_bwd_kernel<<<blocks, kTrainThreads, smem, as_stream(stream)>>>(p);
     TFGK_LAUNCH_CHECK();

@@ -49,12 +49,6 @@ def main():
         gb = (m * k * 4 + nb * m * 128 * 4) / 1e9
         res["proj_nb{}".format(nb)] = {"median_ms": med, "min_ms": best, "algorithmic_gb": gb,
                                       "gbs_at_median": gb / (med * 1e-3), "tf32x3_tflops": 6.0 * m * 104 * 128 * nb / (med * 1e-3) / 1e12}
-    for dbg in (64, 68, 8, 1, 2, 48, 63):          # measurement switches of the kernel: which phase bounds a tile?
-        os.environ["TFGK_PROJ_DEBUG"] = str(dbg)
-        blocks = [(ws[i], bias, ops.ACT_NONE, outs[i]) for i in range(3)]
-        med, best = timed(lambda: ops.gemm_proj(x, blocks), flush=flush)
-        res["proj_nb3_debug{}".format(dbg)] = {"median_ms": med}
-    os.environ.pop("TFGK_PROJ_DEBUG")
     for ctas in (96,):
         blocks = [(ws[i], bias, ops.ACT_NONE, outs[i]) for i in range(3)]
         med, best = timed(lambda: ops.gemm_proj(x, blocks, max_ctas=ctas), flush=flush)

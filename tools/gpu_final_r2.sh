@@ -1,6 +1,6 @@
 #!/bin/bash
 # Round-2 single-GPU validation on a B200 box (run through gpurun): smoke, parity suite, every single-GPU BASELINE config through
-# bench.py, the reference arm, kernel-variant and training timings, launch lists and ncu --set full captures of the hot kernels.
+# bench.py, the reference arm, projection and training timings, launch lists and ncu --set full captures of the hot kernels.
 # Everything lands under gpurun_out/; what should be judged is copied into profiles/ afterwards.
 mkdir -p gpurun_out
 O=gpurun_out
@@ -11,7 +11,6 @@ echo "== reference arm"; timeout 600 python bench.py --impl reference --steps 2 
 for c in cfg1 cfg2 cfg3 cfg4; do
   echo "== bench $c"; timeout 600 python bench.py --config $c --steps 10 --warmup 3 > $O/r2_$c.json 2> $O/r2_$c.err; echo "rc=$?"; cut -c1-160 $O/r2_$c.json
 done
-echo "== kernel variants"; TFGK_BENCH_QUICK=1 timeout 300 python tools/bench_kernels.py > $O/r2_kernel_variants.log 2>&1; cp $O/bench_kernels.json $O/r2_kernel_variants.json; tail -8 $O/r2_kernel_variants.log
 echo "== gemm"; timeout 200 python tools/bench_gemm.py > $O/r2_gemm.log 2>&1; cp $O/bench_gemm.json $O/r2_gemm_proj.json
 echo "== train"; timeout 300 python tools/bench_train.py --steps 5 > $O/r2_train_step.json 2> $O/r2_train.err; cut -c1-300 $O/r2_train_step.json
 if [ "$1" == "--ncu" ]; then
